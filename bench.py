@@ -5,6 +5,7 @@ One "step" = one policy step (10 physics sub-steps + mocap + observation + rewar
 of every environment of the batch.  Contract: see the task statement / DESIGN.md 7.
 
     python bench.py --gpus 1 --steps 512 --warmup 32            # our CUDA engine; also reports configs[2] and [4] as sub-results
+    python bench.py --gpus 1 --steps 512 --warmup 32 --dump-outputs DIR    # ... and what the last timed step returned, for comparing builds
     python bench.py --impl reference --steps 20 --warmup 3      # CPU arm (oracle port; see DESIGN.md 6)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29500 \
         bench.py --gpus 8 ...                                    # env shards, one process per GPU, trajectory gather to rank 0
@@ -53,6 +54,7 @@ ALGO_BYTES = {"pmc": 1676, "epmc": 6208, "epmc_flat": 4672, "sepmc": 9576}
 OBS_W = {"pmc": 207, "epmc": 916, "sepmc": 965}
 ROBOTS_PER_ENV = {"pmc": 1, "epmc": 1, "sepmc": 2}
 ELEMENT = [3]
+DUMP_ROWS = 4096                        # --dump-outputs: at most 3 workloads x 4096 rows x 979 float32 columns, < 64 MB in all
 KERNEL_SOURCES = ["lifelike_agility_and_play_b200/csrc/llq_step16.cuh", "lifelike_agility_and_play_b200/csrc/llq_kernels.cuh", "lifelike_agility_and_play_b200/csrc/llq_cuda.cu",
                   "lifelike_agility_and_play_b200/csrc/llq_math.cuh"]
 
@@ -70,6 +72,11 @@ def parse():
     ap.add_argument("--element", type=int, default=3, help="EPMC element_id (0 flat joystick arena, 1 hurdles, 2 bars, 3 cubes)")
     ap.add_argument("--env", default="pmc", choices=["pmc", "epmc", "sepmc"],
                     help="headline workload: pmc = BASELINE configs[1]; epmc = configs[2] (8192 envs); sepmc = configs[4] (4096 pairs; --envs counts robots)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step of each workload returned (record = obs | action | reward | done as the step kernel "
+                         "writes it into the trajectory slab row, reward, done; with --impl reference: the CPU arm's obs, reward, done) as "
+                         "DIR/<workload>_<name>.npy in float32; rank 0's shard; a workload of more than %d robots is stored as a fixed, "
+                         "seeded sample of %d rows" % (DUMP_ROWS, DUMP_ROWS))
     a = ap.parse_args()
     ELEMENT[0] = a.element
     if a.envs == 0:
@@ -239,27 +246,33 @@ def _cpu_quota():
 def time_cpu_arm(n_envs, steps, warmup, threads=0, env="pmc", repeats=3):
     """Oracle port of the reference step on the host cores (kind 'port': the reference itself is Python over the pybullet wheel,
     which is not installable here -- DESIGN.md 6).  Fixed configuration, no auto-tune: the same batch as the GPU arm per call,
-    one OpenMP thread per CPU of the container's quota.  After a >= 1 s warm-up (OpenMP team up, quota burst spent) `steps`
-    calls are timed `repeats` times; the median is the value, min / max are reported beside it.
-    Returns (median env-steps/s, seconds of the median repeat, threads, envs per call, [rates])."""
+    one OpenMP thread per CPU of the host's quota.  After a >= 1 s spin-up (OpenMP team up, quota burst spent) and max(3, warmup)
+    warm-up calls, `steps` calls are timed `repeats` times; the median is the value, min / max are reported beside it.
+    Returns (median env-steps/s, seconds of the median repeat, threads, envs per call, [rates], (obs, reward, done) of the last call)."""
     quota, _ = _cpu_quota()
     th = threads if threads > 0 else quota
     rpe = ROBOTS_PER_ENV[env]
-    eng = _cpu_engine(n_envs, env, th)
     pool = action_pool_np(n_envs, 8, 5678)
+    # the >= 1 s spin-up takes a wall-clock number of steps, so it runs on an engine of its own; the timed engine takes a fixed
+    # number of warm-up steps and steps the same states from run to run
+    spin = _cpu_engine(n_envs, env, th)
     t_start, k = time.perf_counter(), 0
-    while k < max(3, warmup) or time.perf_counter() - t_start < 1.0:
-        eng.step(pool[k % 8]); k += 1
+    while time.perf_counter() - t_start < 1.0:
+        spin.step(pool[k % 8]); k += 1
+    spin.close()
+    eng = _cpu_engine(n_envs, env, th)
+    for k in range(max(3, warmup)):
+        eng.step(pool[k % 8])
     rates, secs = [], []
     for _ in range(repeats):
         t0 = time.perf_counter()
         for k in range(steps):
-            eng.step(pool[k % 8])
+            last = eng.step(pool[k % 8])
         dt = time.perf_counter() - t0
         secs.append(dt); rates.append((n_envs // rpe) * steps / dt)
     eng.close()
     order = int(np.argsort(rates)[len(rates) // 2])
-    return rates[order], secs[order], th, n_envs, rates
+    return rates[order], secs[order], th, n_envs, rates, last
 
 
 def cpu_baseline_obj(val, cores, n, steps, rates):
@@ -274,7 +287,9 @@ def run_reference(args, rank):
     if rank != 0:
         return
     n = args.cpu_envs if args.env == "pmc" else args.envs
-    val, dt, cores, n, rates = time_cpu_arm(n, args.steps, args.warmup, env=args.env)
+    val, dt, cores, n, rates, (obs, rew, done) = time_cpu_arm(n, args.steps, args.warmup, env=args.env)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(args.env, {"outputs": {"obs": obs, "reward": rew, "done": done.astype(np.float32)}})])
     line = {
         "impl": "reference", "metric": METRIC[args.env], "value": val, "unit": "env-steps/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -337,7 +352,7 @@ def measure(args, env, n, ctx, headline):
         row = (xch.slab() if xch is not None else one_slab)[t]
         # the fused kernel writes the whole record (observation, action, reward, done) straight into the trajectory slab row
         eng.step_device(pool[i % POOL].data_ptr(), row.data_ptr(), reward.data_ptr(), done.data_ptr(), obs_ld=traj_w, stream=stream)
-        state["i"] = i + 1
+        state["i"], state["row"] = i + 1, row
         if t == UNROLL - 1 and do_gather:
             xch.hand_over()                 # unroll complete: it travels on the side stream while the next one is stepped
 
@@ -368,6 +383,11 @@ def measure(args, env, n, ctx, headline):
     wall = time.perf_counter() - wall0
     step_ms = sum(a.elapsed_time(b) for a, b in zip(ev0, ev1))
     c1 = eng.counters()
+    # what the last timed step returned, read before the untimed passes below step the engine again
+    outputs = None
+    if args.dump_outputs:
+        outputs = {"record": state["row"][:, :ow + 14].cpu().numpy(), "reward": reward.cpu().numpy(),
+                   "done": done.cpu().numpy().astype(np.float32)}
 
     # hot (no flush, back-to-back) variant: what a resident rollout loop sees
     h0, h1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -465,7 +485,8 @@ def measure(args, env, n, ctx, headline):
            "e2e_s": e2e_s, "e2e_dev_obs_s": e2e_dev_obs_s, "e2e_steps": e2e_steps, "e2e_pageable": e2e_pageable, "wall": wall,
            "launches": int(c1[4] - c0[4]), "gather": gather, "clocks": sampler.summary() if sampler else None,
            "limit_rows_per_env_substep": float(c1[3] - c0[3]) / max(1, nu * ROBOTS_PER_ENV[env] * args.steps * 10),
-           "contact_rows_per_env_substep": float(c1[2] - c0[2]) / max(1, nu * ROBOTS_PER_ENV[env] * args.steps * 10)}
+           "contact_rows_per_env_substep": float(c1[2] - c0[2]) / max(1, nu * ROBOTS_PER_ENV[env] * args.steps * 10),
+           "outputs": outputs}
     if headline:
         res["actor"] = actor_loop(args, eng, n, ow, ctx, pool, reward, done) if (env == "pmc" and world == 1) else None
     if env != "pmc" and world == 1:
@@ -573,6 +594,16 @@ def hier_actor_loop(args, eng, n, ow, ctx, pool, reward, done, strategic):
     return out
 
 
+def dump_outputs(path, results):
+    """--dump-outputs: DIR/<workload>_<name>.npy for each (workload, per-rank result) pair; the sampled rows depend on the row count only."""
+    os.makedirs(path, exist_ok=True)
+    for key, r in results:
+        n = len(r["outputs"]["reward"])
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False)) if n > DUMP_ROWS else slice(None)
+        for name, a in r["outputs"].items():
+            np.save(os.path.join(path, "%s_%s.npy" % (key, name)), np.ascontiguousarray(a[rows], np.float32))
+
+
 def kernel_name(env):
     inst = {"pmc": 0, "epmc": 1 if ELEMENT[0] == 0 else 3, "sepmc": 2}[env]
     return "llq_step16_kernel<%d>" % inst
@@ -677,6 +708,8 @@ def main():
             dist.destroy_process_group()
         return
 
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(args.env, head)] + list(subs.items()))
     env = args.env
     do_gather = world > 1 and not args.no_gather
     synthetic_inputs()
@@ -716,7 +749,7 @@ def main():
         line[k] = v
     if world == 1:
         cn = args.cpu_envs if env == "pmc" else args.envs
-        cval, cdt, cores, cne, rates = time_cpu_arm(cn, 32, 3, env=env)
+        cval, cdt, cores, cne, rates, _ = time_cpu_arm(cn, 32, 3, env=env)
         line["cpu_baseline"] = cpu_baseline_obj(cval, cores, cne, 32, rates)
     print(json.dumps(line), file=_RESULT_OUT, flush=True)
     if world > 1:

@@ -137,41 +137,3 @@ def test_role_table_points_at_arrays_of_the_right_shape():
     assert [SHAPES[i] for i in hier_role_arrays(False)] == mlc
     assert [SEPMC_SHAPES[i] for i in hier_role_arrays(True)] == mlc + hlc
     assert len(mlc) == 56 and len(mlc + hlc) == 101                      # LLQ_HIER_ROLES_MLC / LLQ_HIER_ROLES_ALL
-
-
-def test_shipped_cube_policy_traverses_the_corridor_on_the_oracle(oracle_lib, blob):
-    """The behavioural pin of DESIGN.md 6 in small: the reference's shipped, Bullet-trained environmental-level policy (cube steps) has to
-    run the corridor of this repo's engine to its end.  Needs the reference's model files; skipped where they are absent (GPU boxes)."""
-    import os
-    import sys
-    path = "/root/reference/data/models/environmental_level_cube.model"
-    if not os.path.exists(path):
-        pytest.skip("reference model files not present")
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
-    from load_reference_model import load
-    from lifelike_agility_and_play_b200 import _capi as capi
-    from lifelike_agility_and_play_b200.sim_envs.playground_env import INIT_STATE_RUN_0, epmc_engine_config
-    pol = EpmcPolicy(load(path).model)
-    erc = {'element_id': 3, 'friction_range': [0.4, 1.0], 'cmd_vary_freq_range': [9999, 10000], 'target_spd_range': [3.0, 3.0],
-           'hole_config': {'min_gap_height': 0.25, 'max_gap_height': 0.25}, 'auxiliary_radius': None, 'disturb_force_config': None}
-    n = 8
-    eng = capi.VecEngine(oracle_lib, n, blob, None, seed=2025, auto_reset=0, **epmc_engine_config(50.0, 50.0, 0.5, 16, 1000, erc))
-    eng.set_init_state(INIT_STATE_RUN_0)
-    obs = eng.reset()
-    state, mask = pol.initial_state(n), np.ones(n, np.float32)
-    reached, fell = 0, 0
-    for t in range(260):
-        act, state = pol.act(obs, state, mask)
-        mask[:] = 0
-        obs, r, d = eng.step(act)
-        if d.any():
-            st, aux = eng.get(capi.F_STATE), eng.get(capi.F_AUX)
-            for i in np.flatnonzero(d):
-                if np.hypot(aux[i, 2] - st[i, 0], aux[i, 3] - st[i, 1]) < 0.5:
-                    reached += 1
-                else:
-                    fell += 1
-            o2 = eng.reset(d.astype(np.uint8))
-            obs = np.where(d[:, None] != 0, o2, obs); mask = d.astype(np.float32)
-    eng.close()
-    assert reached >= 6 and fell <= 1, (reached, fell)          # 8 envs, episodes of 130-200 steps: 7-12 arrivals
