@@ -138,15 +138,15 @@ int launch_step16(llq_handle h, const llq::EnvArrays& E, const float* a, float* 
 int launch_step(llq_handle h, const llq::EnvArrays& E, const float* a, float* obs2, long long ld, cudaStream_t s) {
   const bool epmc = h->cfg.env_kind == LLQ_ENV_EPMC;
   h->counters[4]++;
-  if (epmc && h->cfg.element_id != 0) return launch_step16<3>(h, E, a, obs2, ld, s);      // corridor arenas: the box-aware instance
-  if (h->cfg.env_kind == LLQ_ENV_SEPMC) return launch_step16<2>(h, E, a, obs2, ld, s);
-  return epmc ? launch_step16<1>(h, E, a, obs2, ld, s) : launch_step16<0>(h, E, a, obs2, ld, s);
+  if (epmc && h->cfg.element_id != 0) return launch_step16<llq::kEpmcCorridor>(h, E, a, obs2, ld, s);   // the box-aware instance
+  if (h->cfg.env_kind == LLQ_ENV_SEPMC) return launch_step16<llq::kSepmc>(h, E, a, obs2, ld, s);
+  return epmc ? launch_step16<llq::kEpmcFlat>(h, E, a, obs2, ld, s) : launch_step16<llq::kPmc>(h, E, a, obs2, ld, s);
 }
 void launch_reset(llq_handle h, const llq::EnvArrays& E, const llq::ResetParams& RP, float* obs2, long long ld, cudaStream_t s) {
-  if (h->cfg.env_kind == LLQ_ENV_EPMC && h->cfg.element_id != 0) launch_reset_t<128, 3>(h, E, RP, obs2, ld, s);
-  else if (h->cfg.env_kind == LLQ_ENV_EPMC) launch_reset_t<128, 1>(h, E, RP, obs2, ld, s);
-  else if (h->cfg.env_kind == LLQ_ENV_SEPMC) launch_reset_t<128, 2>(h, E, RP, obs2, ld, s);
-  else launch_reset_t<128, 0>(h, E, RP, obs2, ld, s);
+  if (h->cfg.env_kind == LLQ_ENV_EPMC && h->cfg.element_id != 0) launch_reset_t<128, llq::kEpmcCorridor>(h, E, RP, obs2, ld, s);
+  else if (h->cfg.env_kind == LLQ_ENV_EPMC) launch_reset_t<128, llq::kEpmcFlat>(h, E, RP, obs2, ld, s);
+  else if (h->cfg.env_kind == LLQ_ENV_SEPMC) launch_reset_t<128, llq::kSepmc>(h, E, RP, obs2, ld, s);
+  else launch_reset_t<128, llq::kPmc>(h, E, RP, obs2, ld, s);
   h->counters[4]++;
 }
 
@@ -638,10 +638,8 @@ int llq_get_field(llq_handle h, int field, void* dst) {
       std::vector<double> tmp((size_t)LLQ_AUX_DIM * n);
       CK(cudaMemcpy(tmp.data(), h->E.aux, sizeof(double) * LLQ_AUX_DIM * n, cudaMemcpyDeviceToHost));
       double* o = (double*)dst;
-      for (size_t i = 0; i < n; i++) {
+      for (size_t i = 0; i < n; i++)
         for (int t = 0; t < LLQ_AUX_DIM; t++) o[i * LLQ_AUX_DIM + t] = tmp[(size_t)t * n + i];
-        o[i * LLQ_AUX_DIM + 13] = tmp[13 * n + i];
-      }
       return LLQ_OK;
     }
     case LLQ_F_SAMPLE_PROB:

@@ -16,10 +16,31 @@
 
 namespace llq {
 
-constexpr int kObsDim = 207, kObsDimEpmc = 916, kObsDimSepmc = 965, kPropDim = 33, kActDim = 12, kStateDim = 37, kAuxDim = 18;
-template <int ENV> struct ObsW { static constexpr int value = (ENV == 1 || ENV == 3) ? kObsDimEpmc : (ENV == 2 ? kObsDimSepmc : kObsDim); };
-constexpr int kMaxBoxes = 36, kMaxCand = 12;   // ENV 3 = EPMC corridor (elements 1-3): static boxes per env, contact candidates per step
+// levels, the ENV argument of the kernel templates: the LLQ_ENV_* kinds, with EPMC split into flat ground (element 0) and the
+// corridor arenas of elements 1-3 (static boxes)
+constexpr int kPmc = 0, kEpmcFlat = 1, kSepmc = 2, kEpmcCorridor = 3;
+constexpr int kObsDim = 207, kObsDimEpmc = 916, kObsDimSepmc = 965, kPropDim = 33, kActDim = 12;
+template <int ENV> struct ObsW {
+  static constexpr int value = (ENV == kEpmcFlat || ENV == kEpmcCorridor) ? kObsDimEpmc : (ENV == kSepmc ? kObsDimSepmc : kObsDim);
+};
+constexpr int kMaxBoxes = 36, kMaxCand = 12;   // EPMC corridor: static boxes per env, contact candidates per step
 constexpr int kNewObs = 120;
+// Staging row: kNewObs floats per robot, written by the tail / reset and read by emit_obs_rows.
+//   every level:  prop 33 (joint pos 12 | joint vel 12 | R^T w 3 (24) | R^T v 3 | R[2,:] 3) | action 12 (33)
+//   PMC:          future 72 (45)
+//   EPMC, SEPMC:  R 9 (45, world <- base inertial, row major) | pos 3 (54), then
+//     EPMC:       target direction in the base frame 2 (57) | target speed 1 (59) | |pos| 1 (60) | corridor: yaw 1 (61) | ray masks 3 x 2 (62)
+//     SEPMC:      flag xy 2 (57) | yaw 1 (59) | pad 2 | small vectors 52 (62), see sepmc_pair_tail
+constexpr int kSlotBase = 24, kSlotFuture = 45, kSlotR = 45, kSlotPos = 54;
+constexpr int kSlotTarget = 57, kSlotTargetSpd = 59, kSlotPosLen = 60, kSlotYaw = 61, kSlotMasks = 62;   // EPMC
+constexpr int kSlotFlag = 57, kSlotYawSepmc = 59, kSlotVecs = 62;                                          // SEPMC
+// rows of E.aux, in the order include/llq.h documents for LLQ_F_AUX; SEPMC gives some rows its own names
+namespace aux {
+constexpr int counter = 0, cmd_vary_freq = 1, target_x = 2, target_y = 3, target_spd = 4, target_angle = 5, last_pos_diff_len = 6,
+              total_spd = 7, max_spd = 8, push_count = 9, push_fx = 10, push_fy = 11, push_fz = 12, foot_friction = 13, push_draws = 14,
+              cmd_draws = 15, yaw_accum_deg = 16, init_pos_diff_len = 17;
+constexpr int with_flag = 1, flag_x = 2, flag_y = 3, control_spd = 4, oppo_visible = 5, switch_flag = 6, flag_draws = 15, flag_touch = 17;
+}  // namespace aux
 
 struct DampItem { float m; float c[3]; float Ic[6]; };
 struct JointConst {
@@ -165,10 +186,61 @@ LLQ_DI void epmc_randomize_push(const StepParams& P, unsigned long long seed, lo
   pf[0] = (float)(h * cs); pf[1] = (float)(h * sn); pf[2] = (float)((double)P.pv_lo + u[2] * ((double)P.pv_hi - (double)P.pv_lo));
 }
 
-
-LLQ_DI void push_force_of_draw(const StepParams& P, unsigned long long seed, long long gid, long long ep, int index, float (&pf)[3]) {
-  int d = index;
-  epmc_randomize_push(P, seed, gid, ep, d, pf);
+// ---------------------------------------------------------------------------------------------------------------
+// Pieces of the step tail and the reset that every level shares.
+// Robot state write-back, run on the robot's 4 lanes: this leg's joints and foot (world position), and from lane 0 the base.
+LLQ_DI void store_state(const EnvArrays& E, int N, int env, int k, const float (&q)[3], const float (&qd)[3], V3 foot, double px, double py,
+                        double pz, Q4 qb, V3 lin, V3 ang) {
+  float* sw = E.st;
+#pragma unroll
+  for (int t = 0; t < 3; t++) { sw[(10 + 3 * k + t) * N + env] = q[t]; sw[(22 + 3 * k + t) * N + env] = qd[t]; }
+  E.foot_pos[(3 * k) * N + env] = foot.x; E.foot_pos[(3 * k + 1) * N + env] = foot.y; E.foot_pos[(3 * k + 2) * N + env] = foot.z;
+  if (k == 0) {
+    E.pos[env] = px; E.pos[N + env] = py; E.pos[2 * N + env] = pz;
+    sw[env] = qb.x; sw[N + env] = qb.y; sw[2 * N + env] = qb.z; sw[3 * N + env] = qb.w;
+    sw[4 * N + env] = lin.x; sw[5 * N + env] = lin.y; sw[6 * N + env] = lin.z;
+    sw[7 * N + env] = ang.x; sw[8 * N + env] = ang.y; sw[9 * N + env] = ang.z;
+  }
+}
+// EPMC / SEPMC episode start (LR:115-117): M.init_state with the base yawed by yaw_deg about world z, this leg's joints.  The
+// outputs are references, not one returned struct: with the struct, nvcc 12.9 contracts a product of the reset's foot rotation
+// into a different FMA, and the reset foot positions change in the last bit.
+LLQ_DI Q4 start_pose(const ModelConst& M, int k, double yaw_deg, float (&q)[3], float (&qd)[3], V3& lin, V3& ang) {
+  double sn, cs;
+  sincos(0.5 * yaw_deg * (3.14159265358979323846 / 180.0), &sn, &cs);
+  const float* I0 = M.init_state;
+#pragma unroll
+  for (int i = 0; i < 3; i++) { q[i] = I0[13 + 3 * k + i]; qd[i] = I0[25 + 3 * k + i]; }
+  lin = V3{I0[7], I0[8], I0[9]}; ang = V3{I0[10], I0[11], I0[12]};
+  return qmul(qnormalize(Q4{I0[3], I0[4], I0[5], I0[6]}), Q4{0.f, 0.f, (float)sn, (float)cs});
+}
+// termination on the base orientation (LR:158-179), R = world <- base inertial
+LLQ_DI bool fallen(const M3& R) {
+  const float left_z = R.a02 * R.a10 - R.a12 * R.a00;
+  return left_z > 0.70710678118654752f || left_z < -0.70710678118654752f || R.a22 < 0.5f;
+}
+// prop base block of a staging row (PLE:247-260): R^T w | R^T v | R[2,:]
+LLQ_DI void stage_prop_base(float* snew, const M3& R, V3 ang, V3 lin) {
+  const V3 wl = tmul(R, ang), vl = tmul(R, lin);
+  float* b = snew + kSlotBase;
+  b[0] = wl.x; b[1] = wl.y; b[2] = wl.z; b[3] = vl.x; b[4] = vl.y; b[5] = vl.z;
+  b[6] = R.a20; b[7] = R.a21; b[8] = R.a22;
+}
+// EPMC / SEPMC: the prop base block, then R and pos
+LLQ_DI void stage_pose(float* snew, const M3& R, V3 ang, V3 lin, V3 pos) {
+  stage_prop_base(snew, R, ang, lin);
+  float* r = snew + kSlotR;
+  r[0] = R.a00; r[1] = R.a01; r[2] = R.a02; r[3] = R.a10; r[4] = R.a11; r[5] = R.a12; r[6] = R.a20; r[7] = R.a21; r[8] = R.a22;
+  snew[kSlotPos] = pos.x; snew[kSlotPos + 1] = pos.y; snew[kSlotPos + 2] = pos.z;
+}
+// EPMC staging row on lane 0 of the robot: stage_pose, the direction to the target (dx, dy = target - pos) in the base frame, the
+// target speed and |pos|
+LLQ_DI void stage_epmc(float* snew, const M3& R, V3 ang, V3 lin, double px, double py, double pz, double dx, double dy, float target_spd) {
+  stage_pose(snew, R, ang, lin, V3{(float)px, (float)py, (float)pz});
+  const V3 d = tmul(R, V3{(float)dx, (float)dy, (float)(0.0 - pz)});
+  const float n2 = sqrtf(d.x * d.x + d.y * d.y);
+  snew[kSlotTarget] = d.x / n2; snew[kSlotTarget + 1] = d.y / n2; snew[kSlotTargetSpd] = target_spd;
+  snew[kSlotPosLen] = (float)sqrt(px * px + py * py + pz * pz);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -239,15 +311,14 @@ LLQ_DI void leg_points(const ModelConst& M, const LegConst& L, int k, const floa
   f = rot<1>(f, c2, s2) + ld3(L.j[1].r);
   foot = rot<0>(f, c1, s1) + hip;
 }
-// force of push-randomiser draw `index` (PR:89-99)
 
-// staging row of SEPMC (kNewObs floats per robot): prop 33 | action 12 | R 9 (45) | pos 3 (54) | flag xy 2 (57) | yaw 1 (59) | pad 2 |
-// small vectors 52 (62): percept_vec 5, oppo_info 15, oppo_info_cheat 15, flag_info 7, flag_info_cheat 7, with_flag 2, control_spd 1
+// small vectors of the SEPMC staging row (kSlotVecs): percept_vec 5, oppo_info 15, oppo_info_cheat 15, flag_info 7, flag_info_cheat 7,
+// with_flag 2, control_spd 1
 struct PairState { int with_flag, flag_draws, visible, sw; double flag_x, flag_y; };
 
 // End-of-step pair logic shared by the step and the reset kernels (CTG:495-596, 472-493): visibility, flag switch, the small
-// observation vectors.  Every lane of both robots runs it; `snew` is the robot's staging row, `spart` the partner's.
-template <int PX = 4>   // lane distance of the partner robot: 4 (one robot = 4 lanes) or 16 (one robot = a half-warp)
+// observation vectors.  Every lane of both robots runs it (the partner robot is 4 lanes away); `snew` is the robot's staging row,
+// `spart` the partner's.
 LLQ_DI void sepmc_pair_tail(const ModelConst& M, const LegConst& L, int k, int robot, float* snew, const float* spart, double px, double py,
                             double pz, Q4 qp, Q4 qb, V3 vw, V3 ww, const float (&q)[3], bool touch_own, float fix_spd, unsigned long long seed,
                             long long pair_gid, long long epi, PairState& S) {
@@ -267,11 +338,11 @@ LLQ_DI void sepmc_pair_tail(const ModelConst& M, const LegConst& L, int k, int r
   }
   __syncwarp();
   // partner's root state
-  const double ox = __shfl_xor_sync(FULL, px, PX), oy = __shfl_xor_sync(FULL, py, PX), oz = __shfl_xor_sync(FULL, pz, PX);
-  const Q4 oq = Q4{__shfl_xor_sync(FULL, qb.x, PX), __shfl_xor_sync(FULL, qb.y, PX), __shfl_xor_sync(FULL, qb.z, PX), __shfl_xor_sync(FULL, qb.w, PX)};
-  const V3 ov = V3{__shfl_xor_sync(FULL, vw.x, PX), __shfl_xor_sync(FULL, vw.y, PX), __shfl_xor_sync(FULL, vw.z, PX)};
-  const V3 oww = V3{__shfl_xor_sync(FULL, ww.x, PX), __shfl_xor_sync(FULL, ww.y, PX), __shfl_xor_sync(FULL, ww.z, PX)};
-  const bool touch_other = __shfl_xor_sync(FULL, touch_own ? 1 : 0, PX) != 0;
+  const double ox = __shfl_xor_sync(FULL, px, 4), oy = __shfl_xor_sync(FULL, py, 4), oz = __shfl_xor_sync(FULL, pz, 4);
+  const Q4 oq = Q4{__shfl_xor_sync(FULL, qb.x, 4), __shfl_xor_sync(FULL, qb.y, 4), __shfl_xor_sync(FULL, qb.z, 4), __shfl_xor_sync(FULL, qb.w, 4)};
+  const V3 ov = V3{__shfl_xor_sync(FULL, vw.x, 4), __shfl_xor_sync(FULL, vw.y, 4), __shfl_xor_sync(FULL, vw.z, 4)};
+  const V3 oww = V3{__shfl_xor_sync(FULL, ww.x, 4), __shfl_xor_sync(FULL, ww.y, 4), __shfl_xor_sync(FULL, ww.z, 4)};
+  const bool touch_other = __shfl_xor_sync(FULL, touch_own ? 1 : 0, 4) != 0;
   const V3 opos = V3{(float)ox, (float)oy, (float)oz};
   const float fx = (float)S.flag_x, fy = (float)S.flag_y;
   // visibility (CTG:472-493): the root segment is cast from robot 0 to robot 1 for both agents
@@ -314,18 +385,13 @@ LLQ_DI void sepmc_pair_tail(const ModelConst& M, const LegConst& L, int k, int r
     S.flag_x = -2.0 + 4.0 * u[0]; S.flag_y = -2.0 + 4.0 * u[1];
   }
   if (k == 0) {
-    const V3 wl = tmul(Rq, ww), vl = tmul(Rq, vw);
-    snew[24] = wl.x; snew[25] = wl.y; snew[26] = wl.z; snew[27] = vl.x; snew[28] = vl.y; snew[29] = vl.z;
-    snew[30] = Rq.a20; snew[31] = Rq.a21; snew[32] = Rq.a22;
-    snew[45] = Rq.a00; snew[46] = Rq.a01; snew[47] = Rq.a02; snew[48] = Rq.a10; snew[49] = Rq.a11; snew[50] = Rq.a12;
-    snew[51] = Rq.a20; snew[52] = Rq.a21; snew[53] = Rq.a22;
-    snew[54] = pos.x; snew[55] = pos.y; snew[56] = pos.z;
-    snew[57] = (float)ffx; snew[58] = (float)ffy;                       // the flag where it stood during this step
+    stage_pose(snew, Rq, ww, vw, pos);
+    snew[kSlotFlag] = (float)ffx; snew[kSlotFlag + 1] = (float)ffy;     // the flag where it stood during this step
     const float yaw = atan2f(Rq.a10, Rq.a00);
-    snew[59] = yaw;
+    snew[kSlotYawSepmc] = yaw;
     float sy, cy;
     llq_sincosf(yaw, &sy, &cy);
-    float* v = snew + 62;
+    float* v = snew + kSlotVecs;
     v[0] = pos.x; v[1] = pos.y; v[2] = pos.z; v[3] = cy; v[4] = sy;                          // percept_vec
     const M3 Ro = qmat(qnormalize(oq));
     const float yawo = atan2f(Ro.a10, Ro.a00);
@@ -458,10 +524,11 @@ LLQ_DI void stage_corridor_masks(float* snew, const float* boxes, int nb, int k,
   const unsigned long long mf = box_mask(boxes, nb, k, px, py, pz, 3.35f, false);   // 3 m rays starting up to 0.27 m off the base
   const unsigned long long m1 = box_mask(boxes, nb, k, px, py, pz, 0.f, true);      // horizontal rays at the base height
   if (k == 0) {
-    snew[61] = yaw;
-    snew[62] = __uint_as_float((unsigned)m2); snew[63] = __uint_as_float((unsigned)(m2 >> 32));
-    snew[64] = __uint_as_float((unsigned)mf); snew[65] = __uint_as_float((unsigned)(mf >> 32));
-    snew[66] = __uint_as_float((unsigned)m1); snew[67] = __uint_as_float((unsigned)(m1 >> 32));
+    float* m = snew + kSlotMasks;
+    snew[kSlotYaw] = yaw;
+    m[0] = __uint_as_float((unsigned)m2); m[1] = __uint_as_float((unsigned)(m2 >> 32));
+    m[2] = __uint_as_float((unsigned)mf); m[3] = __uint_as_float((unsigned)(mf >> 32));
+    m[4] = __uint_as_float((unsigned)m1); m[5] = __uint_as_float((unsigned)(m1 >> 32));
   }
 }
 
@@ -491,12 +558,7 @@ LLQ_DI ObsCtx build_obs_new(const MocapDev& mc, const StepParams& P, const Model
   // prop (PLE:247-260): joint_pos | joint_vel | R^T w | R^T v | R[2,:]
 #pragma unroll
   for (int i = 0; i < 3; i++) { snew[3 * lane4 + i] = q[i]; snew[12 + 3 * lane4 + i] = qd[i]; }
-  if (lane4 == 0) {
-    V3 wl = tmul(Rb, ang), vl = tmul(Rb, lin);
-    snew[24] = wl.x; snew[25] = wl.y; snew[26] = wl.z;
-    snew[27] = vl.x; snew[28] = vl.y; snew[29] = vl.z;
-    snew[30] = Rb.a20; snew[31] = Rb.a21; snew[32] = Rb.a22;
-  }
+  if (lane4 == 0) stage_prop_base(snew, Rb, ang, lin);
   // future target `lane4` (ML:75-86, PLE:299-317)
   {
     const double tf = lane4 == 0 ? 1. / 30. : (lane4 == 1 ? 1. / 15. : (lane4 == 2 ? 1. / 3. : 1.));
@@ -509,7 +571,7 @@ LLQ_DI ObsCtx build_obs_new(const MocapDev& mc, const StepParams& P, const Model
     V3 rv = q_rotvec(qnormalize(qmul(qconj(qb), qnormalize(kf.q))));
     float angle = norm3(rv);
     float sc = angle / (angle + 1e-8f);
-    float* o18 = snew + 45 + 18 * lane4;
+    float* o18 = snew + kSlotFuture + 18 * lane4;
     o18[0] = dp.x; o18[1] = dp.y; o18[2] = dp.z;
     o18[3] = sc * rv.x; o18[4] = sc * rv.y; o18[5] = sc * rv.z;
     float ff = (float)ffrac;
@@ -522,11 +584,27 @@ LLQ_DI ObsCtx build_obs_new(const MocapDev& mc, const StepParams& P, const Model
 // Cooperative, coalesced emission of the 8 observation rows owned by this warp.
 // mode 0 (step):  prop = [old[33:99], new] ; prop_a = [old[12:36], act] ; future = new
 // mode 1 (reset): prop = [new, new, new]  ; prop_a = 0                 ; future = new      (PLE:282-290)
-// `do_row` (bit e of a warp-uniform mask) selects which of the 8 rows are written.
+// `do_row` (bit e of a warp-uniform mask) selects which of the 8 rows are written.  EPMC / SEPMC: the perception rays are cast
+// while the row is written.
 constexpr int kHist = 90;   // per-env history carry: prop[33:99] (66) | prop_a[12:36] (24)
 
-// staging row (kNewObs floats per env).  PMC: prop 33 | action 12 | future 72.
-// EPMC: prop 33 | action 12 | R (world<-base inertial, row major) 9 | pos 3 | target 3 | |base_pos| 1   (perception is evaluated while the row is written)
+// Perception ray geometry from the R and pos slots of an EPMC / SEPMC staging row (PGE:409-447).
+// down ray t of percept_2d, over the 25 x 13 grid of 2.4 x 1.2 m in the base frame: its world xy
+LLQ_DI void down_ray_xy(const float* sn, int t, float& x, float& y) {
+  const float* R = sn + kSlotR;
+  const int a = t / 13, b = t - a * 13;
+  const float gx = a == 24 ? 1.2f : -1.2f + (float)a * (2.4f / 24.0f), gy = b == 12 ? 0.6f : -0.6f + (float)b * (1.2f / 12.0f);
+  x = fmaf(R[0], gx, fmaf(R[1], gy, sn[kSlotPos])); y = fmaf(R[3], gx, fmaf(R[4], gy, sn[kSlotPos + 1]));
+}
+// front ray t of percept_front: origins on the 25 x 13 grid over base y in [-0.25, 0.25], z in [-0.3, 0.1]; 3 m along base +x
+LLQ_DI void front_ray(const float* sn, int t, V3& from, V3& d) {
+  const float* R = sn + kSlotR;
+  const int a = t / 13, b = t - a * 13;
+  const float y = a == 24 ? 0.25f : -0.25f + (float)a * (0.5f / 24.0f), z = b == 12 ? 0.1f : -0.3f + (float)b * (0.4f / 12.0f);
+  from = V3{fmaf(R[1], y, fmaf(R[2], z, sn[kSlotPos])), fmaf(R[4], y, fmaf(R[5], z, sn[kSlotPos + 1])),
+            fmaf(R[7], y, fmaf(R[8], z, sn[kSlotPos + 2]))};
+  d = V3{3.f * R[0], 3.f * R[3], 3.f * R[6]};
+}
 template <int ENV, int EPW = 8>   // EPW = envs per warp (8 with 4 lanes per env, 2 with 16)
 LLQ_DI void emit_obs_rows(float* obs, float* obs2, long long obs2_ld, const float* snew_warp, const float* hist_warp, int env0, int n_envs,
                           int mode, unsigned row_mask, const float* boxes_all = nullptr) {
@@ -548,44 +626,41 @@ LLQ_DI void emit_obs_rows(float* obs, float* obs2, long long obs2_ld, const floa
         int a = j - 99;
         if (mode == 1) v = 0.f;
         else v = a < 24 ? hs[66 + a] : sn[kPropDim + a - 24];
-      } else if (ENV == 0) {
-        v = sn[45 + (j - 135)];
-      } else if (ENV == 3) {
+      } else if (ENV == kPmc) {
+        v = sn[kSlotFuture + (j - 135)];
+      } else if (ENV == kEpmcCorridor) {
         // EPMC corridor perception against the ground slab and the env's candidate boxes (PGE:374-447)
-        const V3 pos = V3{sn[54], sn[55], sn[56]};
+        const V3 pos = ld3(sn + kSlotPos);
         const float* bxs = boxes_all + (size_t)(env0 + e) * (6 * kMaxBoxes);
+        const float* ms = sn + kSlotMasks;
         if (j < 460) {
-          const unsigned long long m = ((unsigned long long)__float_as_uint(sn[63]) << 32) | __float_as_uint(sn[62]);
-          const int t = j - 135, a = t / 13, b = t - a * 13;
-          const float gx = a == 24 ? 1.2f : -1.2f + (float)a * (2.4f / 24.0f), gy = b == 12 ? 0.6f : -0.6f + (float)b * (1.2f / 12.0f);
-          const float x = fmaf(sn[45], gx, fmaf(sn[46], gy, pos.x)), y = fmaf(sn[48], gx, fmaf(sn[49], gy, pos.y));
+          const unsigned long long m = ((unsigned long long)__float_as_uint(ms[1]) << 32) | __float_as_uint(ms[0]);
+          float x, y;
+          down_ray_xy(sn, j - 135, x, y);
           v = fmaxf(down_ray_top(x, y, bxs, m), 0.f);          // hit z of the down ray (0 when it misses everything)
         } else if (j < 588) {
-          const unsigned long long m = ((unsigned long long)__float_as_uint(sn[67]) << 32) | __float_as_uint(sn[66]);
-          const float ang = sn[61] + 6.283185307179586f * (float)(j - 460) * (1.0f / 128.0f);
+          const unsigned long long m = ((unsigned long long)__float_as_uint(ms[5]) << 32) | __float_as_uint(ms[4]);
+          const float ang = sn[kSlotYaw] + 6.283185307179586f * (float)(j - 460) * (1.0f / 128.0f);
           float sa, ca;
           llq_sincosf(ang, &sa, &ca);
           const float f = ray_boxlist(pos, V3{20.f * ca, 20.f * sa, 0.f}, bxs, m);
-          v = f < 0.f ? sn[60] : f * 20.f * sqrtf(ca * ca + sa * sa);
+          v = f < 0.f ? sn[kSlotPosLen] : f * 20.f * sqrtf(ca * ca + sa * sa);
         } else if (j < 913) {
-          const unsigned long long m = ((unsigned long long)__float_as_uint(sn[65]) << 32) | __float_as_uint(sn[64]);
-          const int t = j - 588, a = t / 13, b = t - a * 13;
-          const float y = a == 24 ? 0.25f : -0.25f + (float)a * (0.5f / 24.0f), z = b == 12 ? 0.1f : -0.3f + (float)b * (0.4f / 12.0f);
-          const V3 from = V3{fmaf(sn[46], y, fmaf(sn[47], z, pos.x)), fmaf(sn[49], y, fmaf(sn[50], z, pos.y)), fmaf(sn[52], y, fmaf(sn[53], z, pos.z))};
-          const V3 d = V3{3.f * sn[45], 3.f * sn[48], 3.f * sn[51]};
+          const unsigned long long m = ((unsigned long long)__float_as_uint(ms[3]) << 32) | __float_as_uint(ms[2]);
+          V3 from, d;
+          front_ray(sn, j - 588, from, d);
           const float f = ray_boxlist(from, d, bxs, m);
           v = (f < 0.f ? 1.f : f) * norm3(d);
         } else {
-          v = sn[57 + (j - 913)];
+          v = sn[kSlotTarget + (j - 913)];
         }
-      } else if (ENV == 2) {
+      } else if (ENV == kSepmc) {
         // SEPMC perception against ground slab, walls and flag (CTG:598-638, PGE:22-54)
-        const V3 pos = V3{sn[54], sn[55], sn[56]};
-        const float fx = sn[57], fy = sn[58];
+        const V3 pos = ld3(sn + kSlotPos);
+        const float fx = sn[kSlotFlag], fy = sn[kSlotFlag + 1];
         if (j < 460) {                             // percept_2d: down rays over the 25 x 13 grid in the full base frame, value = hit z
-          const int t = j - 135, a = t / 13, b = t - a * 13;
-          const float gx = a == 24 ? 1.2f : -1.2f + (float)a * (2.4f / 24.0f), gy = b == 12 ? 0.6f : -0.6f + (float)b * (1.2f / 12.0f);
-          const float x = fmaf(sn[45], gx, fmaf(sn[46], gy, pos.x)), y = fmaf(sn[48], gx, fmaf(sn[49], gy, pos.y));
+          float x, y;
+          down_ray_xy(sn, j - 135, x, y);
           // a vertical ray sees the highest top among the boxes whose footprint holds (x, y): flag 0.5, walls 2, ground 0
           const bool in_x = fabsf(x) <= 2.5f, in_y = fabsf(y) <= 2.5f;
           const bool wall = (in_x && fabsf(fabsf(y) - 2.5f) <= 0.005f) || (in_y && fabsf(fabsf(x) - 2.5f) <= 0.005f);
@@ -596,7 +671,7 @@ LLQ_DI void emit_obs_rows(float* obs, float* obs2, long long obs2_ld, const floa
             v = f < 0.f ? 0.f : fmaf(f, -20.f, 10.f);
           }
         } else if (j < 588) {                      // percept_1d: 128 horizontal rays of 20 m; a miss reports |ray_from|
-          const float ang = sn[59] + 6.283185307179586f * (float)(j - 460) * (1.0f / 128.0f);
+          const float ang = sn[kSlotYawSepmc] + 6.283185307179586f * (float)(j - 460) * (1.0f / 128.0f);
           float sa, ca;
           llq_sincosf(ang, &sa, &ca);
           const V3 d = V3{20.f * ca, 20.f * sa, 0.f};
@@ -604,31 +679,30 @@ LLQ_DI void emit_obs_rows(float* obs, float* obs2, long long obs2_ld, const floa
           const float f = inside ? ray_arena_inside(pos, d, fx, fy) : ray_arena(pos, d, fx, fy);
           v = f < 0.f ? norm3(pos) : f * 20.f * sqrtf(ca * ca + sa * sa);
         } else if (j < 913) {                      // percept_front: 25 x 13 rays of 3 m along body +x; a miss reports 3
-          const int t = j - 588, a = t / 13, b = t - a * 13;
-          const float y = a == 24 ? 0.25f : -0.25f + (float)a * (0.5f / 24.0f), z = b == 12 ? 0.1f : -0.3f + (float)b * (0.4f / 12.0f);
-          const V3 from = V3{fmaf(sn[46], y, fmaf(sn[47], z, pos.x)), fmaf(sn[49], y, fmaf(sn[50], z, pos.y)), fmaf(sn[52], y, fmaf(sn[53], z, pos.z))};
-          const V3 d = V3{3.f * sn[45], 3.f * sn[48], 3.f * sn[51]};
+          V3 from, d;
+          front_ray(sn, j - 588, from, d);
           const bool inside = fabsf(from.x) < 2.49f && fabsf(from.y) < 2.49f && from.z > 0.f;
           const float f = inside ? ray_arena_inside(from, d, fx, fy) : ray_arena(from, d, fx, fy);
           v = (f < 0.f ? 1.f : f) * norm3(d);
         } else {
-          v = sn[62 + (j - 913)];
+          v = sn[kSlotVecs + (j - 913)];
         }
       } else if (j < 460) {
         v = 0.f;                                   // percep_2d: every down-ray hits the slab top, hit z = 0 (PGE:431-447)
       } else if (j < 588) {
-        v = sn[60];                                // percep_1d: horizontal rays miss => |ray_from| (PGE:49-53,388-394)
+        v = sn[kSlotPosLen];                       // percep_1d: horizontal rays miss => |ray_from| (PGE:49-53,388-394)
       } else if (j < 913) {                        // percep_front (PGE:409-429) against the ground slab
+        const float* R = sn + kSlotR;
         int t = j - 588, i = t / 13, jj = t - i * 13;
         float y = i == 24 ? 0.25f : -0.25f + (float)i * (0.5f / 24.0f);
         float z = jj == 12 ? 0.1f : -0.3f + (float)jj * (0.4f / 12.0f);
-        float fz = fmaf(sn[52], y, fmaf(sn[53], z, sn[56]));          // from.z = R[2,1] y + R[2,2] z + pos.z
-        float dz = 3.0f * sn[51];                                     // (to - from).z = 3 R[2,0]
-        float len = 3.0f * sqrtf(sn[45] * sn[45] + sn[48] * sn[48] + sn[51] * sn[51]);
+        float fz = fmaf(R[7], y, fmaf(R[8], z, sn[kSlotPos + 2]));   // from.z = R[2,1] y + R[2,2] z + pos.z
+        float dz = 3.0f * R[6];                                       // (to - from).z = 3 R[2,0]
+        float len = 3.0f * sqrtf(R[0] * R[0] + R[3] * R[3] + R[6] * R[6]);
         float tz = fz + dz;
         v = (fz > 0.f && tz < 0.f) ? len * (fz / (fz - tz)) : len;
       } else {
-        v = sn[57 + (j - 913)];
+        v = sn[kSlotTarget + (j - 913)];
       }
       obs[(size_t)(env0 + e) * OW + j] = v;
       if (obs2) obs2[(size_t)(env0 + e) * obs2_ld + j] = v;
@@ -732,12 +806,12 @@ __global__ void __launch_bounds__(BLOCK) pmc_reset_kernel(EnvArrays E, MocapDev 
   bool doit = valid;
   if (RP.mode == 3) doit = false;
   else if (RP.mode == 0) doit = doit && E.done[env] != 0;
-  else if (RP.mask) doit = doit && (RP.mask[env] != 0 || (ENV == 2 && RP.mask[env ^ 1] != 0));   // SEPMC: a pair resets as a whole
+  else if (RP.mask) doit = doit && (RP.mask[env] != 0 || (ENV == kSepmc && RP.mask[env ^ 1] != 0));   // SEPMC: a pair resets as a whole
   const unsigned wm = __ballot_sync(FULL, doit);
   if (wm == 0) return;                                   // warp-uniform: nothing to reset in these 8 envs
   const LegConst& L = M.leg[k];
 
-  if (ENV == 2) {
+  if (ENV == kSepmc) {
     // ---------------- SEPMC reset (CTG:261-304, 204-230); draws keyed by the pair: stream 1 = [fix_spd, with_flag, friction, x0 |
     // y0, x1, y1, yaw0 | yaw1, flag x, flag y]
     const int robot = env & 1;
@@ -752,22 +826,16 @@ __global__ void __launch_bounds__(BLOCK) pmc_reset_kernel(EnvArrays E, MocapDev 
     const double foot_mu = (double)P.fr_lo + u0[2] * ((double)P.fr_hi - (double)P.fr_lo);
     const double px = robot == 0 ? -2.0 + 4.0 * u0[3] : -2.0 + 4.0 * u1[1], py = robot == 0 ? -2.0 + 4.0 * u1[0] : -2.0 + 4.0 * u1[2];
     // both robots are handed the same mutable init dict => one running yaw for the pair (CTG:209-215)
-    const double acc0 = E.aux[16 * N + (env & ~1)];
+    const double acc0 = E.aux[aux::yaw_accum_deg * N + (env & ~1)];
     const double yaw_a = fmod(acc0 + 360.0 * u1[3], 360.0), yaw_b = fmod(yaw_a + 360.0 * u2[0], 360.0);
-    const double yaw_deg = robot == 0 ? yaw_a : yaw_b;
-    double sn, cs;
-    sincos(0.5 * yaw_deg * (3.14159265358979323846 / 180.0), &sn, &cs);
-    const float* I0 = M.init_state;
-    const Q4 qn = qmul(qnormalize(Q4{I0[3], I0[4], I0[5], I0[6]}), Q4{0.f, 0.f, (float)sn, (float)cs});
     float q[3], qd[3];
-#pragma unroll
-    for (int i = 0; i < 3; i++) { q[i] = I0[13 + 3 * k + i]; qd[i] = I0[25 + 3 * k + i]; }
-    const V3 lin = V3{I0[7], I0[8], I0[9]}, ang = V3{I0[10], I0[11], I0[12]};
+    V3 lin, ang;
+    const Q4 qn = start_pose(M, k, robot == 0 ? yaw_a : yaw_b, q, qd, lin, ang);
     const Q4 qI = Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]};
     const Q4 qp = qmul(qnormalize(qn), qconj(qI));
     PairState PS = {robot == 0 ? wflag : 1 - wflag, 0, 1, 0, -2.0 + 4.0 * u2[1], -2.0 + 4.0 * u2[2]};
     // reset() runs _prepare_drill too (CTG:302): its flag-switch test reads the stale manifolds of the previous episode's last step
-    const bool touch_own = E.aux[17 * N + env] != 0.0;
+    const bool touch_own = E.aux[aux::flag_touch * N + env] != 0.0;
     float* snew = &s_new[threadIdx.x >> 2][0];
     const float* spart = &s_new[(threadIdx.x >> 2) ^ 1][0];
     sepmc_pair_tail(M, L, k, robot, snew, spart, px, py, 0.5, qp, qn, lin, ang, q, touch_own, fix_spd, RP.seed, gid, ep, PS);
@@ -777,26 +845,22 @@ __global__ void __launch_bounds__(BLOCK) pmc_reset_kernel(EnvArrays E, MocapDev 
     float pf[3] = {0.f, 0.f, 0.f};
     if (P.push_enabled) push_draws = 1;                              // PR:52-54: draw #0 becomes the current _randomized_force
     if (doit) {
-      float* sw = E.st;
-      V3 f = mul(qmat(qp), foot_in_base(L, q[0], q[1], q[2]));
-#pragma unroll
-      for (int i = 0; i < 3; i++) { sw[(10 + 3 * k + i) * N + env] = q[i]; sw[(22 + 3 * k + i) * N + env] = qd[i]; }
+      const V3 f = mul(qmat(qp), foot_in_base(L, q[0], q[1], q[2]));
+      store_state(E, N, env, k, q, qd, V3{(float)px + f.x, (float)py + f.y, 0.5f + f.z}, px, py, 0.5, qn, lin, ang);
       E.warm[k * N + env] = 0.f;
-      E.foot_pos[(3 * k) * N + env] = (float)px + f.x; E.foot_pos[(3 * k + 1) * N + env] = (float)py + f.y; E.foot_pos[(3 * k + 2) * N + env] = 0.5f + f.z;
       if (k == 0) {
-        E.pos[env] = px; E.pos[N + env] = py; E.pos[2 * N + env] = 0.5;
-        float b[10] = {qn.x, qn.y, qn.z, qn.w, lin.x, lin.y, lin.z, ang.x, ang.y, ang.z};
-#pragma unroll
-        for (int i = 0; i < 10; i++) sw[i * N + env] = b[i];
         E.time[env] = 0.0; E.reward_sum[env] = 0.f; E.episode_steps[env] = 0; E.episode[env] = ep + 1;
         double* A = E.aux;
-        A[env] = 0; A[N + env] = PS.with_flag; A[2 * N + env] = PS.flag_x; A[3 * N + env] = PS.flag_y; A[4 * N + env] = fix_spd;
-        A[5 * N + env] = PS.visible; A[6 * N + env] = PS.sw; A[7 * N + env] = 0.0; A[8 * N + env] = 0.0; A[9 * N + env] = P.push_start_count;
-        A[10 * N + env] = pf[0]; A[11 * N + env] = pf[1]; A[12 * N + env] = pf[2]; A[13 * N + env] = foot_mu; A[14 * N + env] = push_draws;
-        A[15 * N + env] = PS.flag_draws; A[16 * N + env] = yaw_b; A[17 * N + env] = touch_own ? 1.0 : 0.0;
+        A[aux::counter * N + env] = 0; A[aux::with_flag * N + env] = PS.with_flag; A[aux::flag_x * N + env] = PS.flag_x;
+        A[aux::flag_y * N + env] = PS.flag_y; A[aux::control_spd * N + env] = fix_spd; A[aux::oppo_visible * N + env] = PS.visible;
+        A[aux::switch_flag * N + env] = PS.sw; A[aux::total_spd * N + env] = 0.0; A[aux::max_spd * N + env] = 0.0;
+        A[aux::push_count * N + env] = P.push_start_count;
+        A[aux::push_fx * N + env] = pf[0]; A[aux::push_fy * N + env] = pf[1]; A[aux::push_fz * N + env] = pf[2];
+        A[aux::foot_friction * N + env] = foot_mu; A[aux::push_draws * N + env] = push_draws; A[aux::flag_draws * N + env] = PS.flag_draws;
+        A[aux::yaw_accum_deg * N + env] = yaw_b; A[aux::flag_touch * N + env] = touch_own ? 1.0 : 0.0;
       }
     }
-  } else if (ENV == 1 || ENV == 3) {
+  } else if (ENV == kEpmcFlat || ENV == kEpmcCorridor) {
     // ---------------- EPMC reset (PGE:196-249)
     long long ep = E.episode[env];
     const long long gid = RP.gid0 + env;
@@ -807,59 +871,40 @@ __global__ void __launch_bounds__(BLOCK) pmc_reset_kernel(EnvArrays E, MocapDev 
     float pf[3] = {0.f, 0.f, 0.f};
     if (P.push_enabled) epmc_randomize_push(P, RP.seed, gid, ep, push_draws, pf);                          // PR:52-54
     const int cmd_freq = P.cmd_freq_lo + (int)floor(u[2] * (double)(P.cmd_freq_hi - P.cmd_freq_lo));       // PGE:223
-    const double yaw_deg = fmod(E.aux[16 * N + env] + 360.0 * u[1], 360.0);                                // PGE:181-189 (accumulates)
-    double sn, cs;
-    sincos(0.5 * yaw_deg * (3.14159265358979323846 / 180.0), &sn, &cs);
-    const float* I0 = M.init_state;
-    const Q4 qn = qmul(qnormalize(Q4{I0[3], I0[4], I0[5], I0[6]}), Q4{0.f, 0.f, (float)sn, (float)cs});
+    const double yaw_deg = fmod(E.aux[aux::yaw_accum_deg * N + env] + 360.0 * u[1], 360.0);                 // PGE:181-189 (accumulates)
     float q[3], qd[3];
-#pragma unroll
-    for (int i = 0; i < 3; i++) { q[i] = I0[13 + 3 * k + i]; qd[i] = I0[25 + 3 * k + i]; }
-    const V3 lin = V3{I0[7], I0[8], I0[9]}, ang = V3{I0[10], I0[11], I0[12]};
+    V3 lin, ang;
+    const Q4 qn = start_pose(M, k, yaw_deg, q, qd, lin, ang);
     float* snew = &s_new[threadIdx.x >> 2][0];
     const M3 Rq = qmat(qnormalize(qn));
-    const float target_spd = (float)E.aux[4 * N + env];            // persists across episodes (PGE:170-172)
+    const float target_spd = (float)E.aux[aux::target_spd * N + env];   // persists across episodes (PGE:170-172)
     double tgx0 = 8.0;
     int nb0 = 0;
-    if (ENV == 3) nb0 = generate_corridor(P, RP.seed, gid, ep, E.boxes + (size_t)env * (6 * kMaxBoxes), doit && k == 0, tgx0);   // PGE:216-219
+    if (ENV == kEpmcCorridor) nb0 = generate_corridor(P, RP.seed, gid, ep, E.boxes + (size_t)env * (6 * kMaxBoxes), doit && k == 0, tgx0);   // PGE:216-219
 #pragma unroll
     for (int i = 0; i < 3; i++) { snew[3 * k + i] = q[i]; snew[12 + 3 * k + i] = qd[i]; }
-    if (k == 0) {
-      V3 wl = tmul(Rq, ang), vl = tmul(Rq, lin);
-      snew[24] = wl.x; snew[25] = wl.y; snew[26] = wl.z; snew[27] = vl.x; snew[28] = vl.y; snew[29] = vl.z;
-      snew[30] = Rq.a20; snew[31] = Rq.a21; snew[32] = Rq.a22;
-      snew[45] = Rq.a00; snew[46] = Rq.a01; snew[47] = Rq.a02; snew[48] = Rq.a10; snew[49] = Rq.a11; snew[50] = Rq.a12;
-      snew[51] = Rq.a20; snew[52] = Rq.a21; snew[53] = Rq.a22;
-      snew[54] = 0.f; snew[55] = 0.f; snew[56] = 0.5f;
-      V3 d = tmul(Rq, V3{(float)tgx0, 0.f, -0.5f});                 // target - pos (0,0,0.5); element 0: (8,0,0) (BSE:247-248)
-      float n2 = sqrtf(d.x * d.x + d.y * d.y);
-      snew[57] = d.x / n2; snew[58] = d.y / n2; snew[59] = target_spd;
-      snew[60] = 0.5f;
-    }
-    if (ENV == 3) {
+    // the tail's row at pos (0, 0, 0.5) with target (tgx0, 0); element 0: (8, 0) (BSE:247-248)
+    if (k == 0) stage_epmc(snew, Rq, ang, lin, 0.0, 0.0, 0.5, tgx0, 0.0, target_spd);
+    if (ENV == kEpmcCorridor) {
       __syncwarp();                                                 // lane 0's boxes are visible to the env's other lanes
       stage_corridor_masks(snew, E.boxes + (size_t)env * (6 * kMaxBoxes), doit ? nb0 : E.nbox[env], k, 0.f, 0.f, 0.5f, atan2f(Rq.a10, Rq.a00));
     }
     if (doit) {
-      float* sw = E.st;
       const Q4 qI = Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]};
-      V3 f = mul(qmat(qmul(qnormalize(qn), qconj(qI))), foot_in_base(L, q[0], q[1], q[2]));
-#pragma unroll
-      for (int i = 0; i < 3; i++) { sw[(10 + 3 * k + i) * N + env] = q[i]; sw[(22 + 3 * k + i) * N + env] = qd[i]; }
+      const V3 f = mul(qmat(qmul(qnormalize(qn), qconj(qI))), foot_in_base(L, q[0], q[1], q[2]));
       E.warm[k * N + env] = 0.f;
-      E.foot_pos[(3 * k) * N + env] = f.x; E.foot_pos[(3 * k + 1) * N + env] = f.y; E.foot_pos[(3 * k + 2) * N + env] = 0.5f + f.z;
+      store_state(E, N, env, k, q, qd, V3{f.x, f.y, 0.5f + f.z}, 0.0, 0.0, 0.5, qn, lin, ang);
       if (k == 0) {
-        E.pos[env] = 0.0; E.pos[N + env] = 0.0; E.pos[2 * N + env] = 0.5;
-        float b[10] = {qn.x, qn.y, qn.z, qn.w, lin.x, lin.y, lin.z, ang.x, ang.y, ang.z};
-#pragma unroll
-        for (int i = 0; i < 10; i++) sw[i * N + env] = b[i];
         E.time[env] = 0.0; E.reward_sum[env] = 0.f; E.episode_steps[env] = 0; E.episode[env] = ep + 1;
         double* A = E.aux;
-        A[env] = 0; A[N + env] = cmd_freq; A[2 * N + env] = tgx0; A[3 * N + env] = 0.0; A[6 * N + env] = fabs(tgx0); A[7 * N + env] = 0.0;
-        A[17 * N + env] = fabs(tgx0);                                  // init_pos_diff_len (PGE:192-195)
-        if (ENV == 3) E.nbox[env] = nb0;
-        A[8 * N + env] = 0.0; A[9 * N + env] = P.push_start_count; A[10 * N + env] = pf[0]; A[11 * N + env] = pf[1]; A[12 * N + env] = pf[2];
-        A[13 * N + env] = foot_mu; A[14 * N + env] = push_draws; A[15 * N + env] = 0; A[16 * N + env] = yaw_deg;
+        A[aux::counter * N + env] = 0; A[aux::cmd_vary_freq * N + env] = cmd_freq; A[aux::target_x * N + env] = tgx0;
+        A[aux::target_y * N + env] = 0.0; A[aux::last_pos_diff_len * N + env] = fabs(tgx0); A[aux::total_spd * N + env] = 0.0;
+        A[aux::init_pos_diff_len * N + env] = fabs(tgx0);                                                   // PGE:192-195
+        if (ENV == kEpmcCorridor) E.nbox[env] = nb0;
+        A[aux::max_spd * N + env] = 0.0; A[aux::push_count * N + env] = P.push_start_count;
+        A[aux::push_fx * N + env] = pf[0]; A[aux::push_fy * N + env] = pf[1]; A[aux::push_fz * N + env] = pf[2];
+        A[aux::foot_friction * N + env] = foot_mu; A[aux::push_draws * N + env] = push_draws; A[aux::cmd_draws * N + env] = 0;
+        A[aux::yaw_accum_deg * N + env] = yaw_deg;
       }
     }
   } else {
@@ -899,22 +944,14 @@ __global__ void __launch_bounds__(BLOCK) pmc_reset_kernel(EnvArrays E, MocapDev 
   float* snew = &s_new[threadIdx.x >> 2][0];
   build_obs_new(mc, P, M, k, clip, frame_id, frac, kb.px, kb.py, kb.pz, kb.q, kb.lin, kb.ang, q, qd, snew);
   if (doit) {
-    float* sw = E.st;
     const Q4 qI = Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]};
-    V3 f = mul(qmat(qmul(qnormalize(kb.q), qconj(qI))), foot_in_base(L, q[0], q[1], q[2]));
+    const V3 f = mul(qmat(qmul(qnormalize(kb.q), qconj(qI))), foot_in_base(L, q[0], q[1], q[2]));
+    store_state(E, N, env, k, q, qd, V3{(float)kb.px + f.x, (float)kb.py + f.y, (float)kb.pz + f.z}, kb.px, kb.py, kb.pz, kb.q, kb.lin, kb.ang);
 #pragma unroll
-    for (int i = 0; i < 3; i++) {
-      sw[(10 + 3 * k + i) * N + env] = q[i]; sw[(22 + 3 * k + i) * N + env] = qd[i];
-      E.kin[(13 + 3 * k + i) * N + env] = q[i]; E.kin[(25 + 3 * k + i) * N + env] = qd[i];
-    }
+    for (int i = 0; i < 3; i++) { E.kin[(13 + 3 * k + i) * N + env] = q[i]; E.kin[(25 + 3 * k + i) * N + env] = qd[i]; }
     E.warm[k * N + env] = 0.f;
-    E.foot_pos[(3 * k) * N + env] = (float)kb.px + f.x; E.foot_pos[(3 * k + 1) * N + env] = (float)kb.py + f.y;
-    E.foot_pos[(3 * k + 2) * N + env] = (float)kb.pz + f.z;
     if (k == 0) {
-      E.pos[env] = kb.px; E.pos[N + env] = kb.py; E.pos[2 * N + env] = kb.pz;
-      float b[13] = {kb.q.x, kb.q.y, kb.q.z, kb.q.w, kb.lin.x, kb.lin.y, kb.lin.z, kb.ang.x, kb.ang.y, kb.ang.z, 0.f, 0.f, 0.f};
-#pragma unroll
-      for (int i = 0; i < 10; i++) sw[i * N + env] = b[i];
+      const float b[10] = {kb.q.x, kb.q.y, kb.q.z, kb.q.w, kb.lin.x, kb.lin.y, kb.lin.z, kb.ang.x, kb.ang.y, kb.ang.z};
       E.kin[env] = (float)kb.px; E.kin[N + env] = (float)kb.py; E.kin[2 * N + env] = (float)kb.pz;
 #pragma unroll
       for (int i = 0; i < 10; i++) E.kin[(3 + i) * N + env] = b[i];

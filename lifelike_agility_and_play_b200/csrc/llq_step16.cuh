@@ -421,8 +421,8 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
   float q[3], qd[3];
 #pragma unroll
   for (int t = 0; t < 3; t++) { q[t] = T.q[3 * k + t]; qd[t] = T.qd[3 * k + t]; }
-  const int clip = ENV == 0 ? E.clip[env] : 0;
-  const long long epi = ENV != 0 ? E.episode[env] - 1 : 0;
+  const int clip = ENV == kPmc ? E.clip[env] : 0;
+  const long long epi = ENV != kPmc ? E.episode[env] - 1 : 0;
   const int robot = env & 1;
   const long long pair_gid = gid0 + (env & ~1);
   bool done = false;
@@ -432,7 +432,7 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
   const Q4 qI = Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]};
   Q4 qb;
   PairState PS = {0, 0, 1, 0, 0.0, 0.0};
-  if (ENV == 0) {
+  if (ENV == kPmc) {
     qb = qmul(qp, qI);                                 // back to the pybullet (inertial-frame) convention
     float* snew = s_new + el * kNewObs;
     ObsCtx oc = build_obs_new(mc, P, M, k, clip, frame_id, frame_frac, px, py, pz, qb, vw, ww, q, qd, snew);
@@ -462,9 +462,7 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
     float rew = P.w_jp * expf(-1.0f * djp) + P.w_jv * expf(-0.1f * djv) + P.w_ee * expf(-40.0f * dee) +
                 P.w_pose * expf(-20.0f * dp - 10.0f * angle * angle) + P.w_vel * expf(-2.0f * dot(dvl3, dvl3) - 0.2f * dot(dva3, dva3));
     // termination (PLE:337-348, LR:158-179, ML:168-172)
-    M3 Rq = qmat(q1);
-    float left_z = Rq.a02 * Rq.a10 - Rq.a12 * Rq.a00;
-    bool fall = left_z > 0.70710678118654752f || left_z < -0.70710678118654752f || Rq.a22 < 0.5f;
+    bool fall = fallen(qmat(q1));
     int nf = mc.clip_off[clip + 1] - mc.clip_off[clip];
     bool ended = frame_id >= nf - P.margin - 1;
     bool diff = fabsf(angle) > 1.0f || dp > 1.0f;
@@ -480,58 +478,40 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
     done = fall || ended || diff || ob_hit || bad;                                     // PLE:347
     rew_out = rew;
     if (wr) {
-      float* sw = E.st;
+      store_state(E, N, env, k, q, qd, fd, px, py, pz, qb, vw, ww);
 #pragma unroll
-      for (int t = 0; t < 3; t++) {
-        sw[(10 + 3 * k + t) * N + env] = q[t];
-        sw[(22 + 3 * k + t) * N + env] = qd[t];
-        E.kin[(13 + 3 * k + t) * N + env] = oc.kq[t];
-        E.kin[(25 + 3 * k + t) * N + env] = oc.kqd[t];
-      }
-      E.foot_pos[(3 * k) * N + env] = fd.x; E.foot_pos[(3 * k + 1) * N + env] = fd.y; E.foot_pos[(3 * k + 2) * N + env] = fd.z;
+      for (int t = 0; t < 3; t++) { E.kin[(13 + 3 * k + t) * N + env] = oc.kq[t]; E.kin[(25 + 3 * k + t) * N + env] = oc.kqd[t]; }
       if (k == 0) {
-        E.pos[env] = px; E.pos[N + env] = py; E.pos[2 * N + env] = pz;
-        sw[env] = qb.x; sw[N + env] = qb.y; sw[2 * N + env] = qb.z; sw[3 * N + env] = qb.w;
-        sw[4 * N + env] = vw.x; sw[5 * N + env] = vw.y; sw[6 * N + env] = vw.z;
-        sw[7 * N + env] = ww.x; sw[8 * N + env] = ww.y; sw[9 * N + env] = ww.z;
-        E.time[env] = time;
         if (P.has_ob) E.ob_id[env] = ob_id;
-        float rs = E.reward_sum[env] + rew;
-        E.reward_sum[env] = rs;
-        E.episode_steps[env] += 1;
-        E.reward[env] = rew;
-        E.done[env] = done ? 1 : 0;
         E.kin[env] = (float)oc.kb.px; E.kin[N + env] = (float)oc.kb.py; E.kin[2 * N + env] = (float)oc.kb.pz;
         E.kin[3 * N + env] = oc.kb.q.x; E.kin[4 * N + env] = oc.kb.q.y; E.kin[5 * N + env] = oc.kb.q.z; E.kin[6 * N + env] = oc.kb.q.w;
         E.kin[7 * N + env] = oc.kb.lin.x; E.kin[8 * N + env] = oc.kb.lin.y; E.kin[9 * N + env] = oc.kb.lin.z;
         E.kin[10 * N + env] = oc.kb.ang.x; E.kin[11 * N + env] = oc.kb.ang.y; E.kin[12 * N + env] = oc.kb.ang.z;
         if (done) {
-          E.done_reward[env] = rs;
+          E.done_reward[env] = E.reward_sum[env] + rew;
           atomicMax(&winner[clip], env);       // highest finished env index owns the clip's slot this step (PLE:236)
         }
       }
     }
-  } else if (ENV == 2) {
+  } else if (ENV == kSepmc) {
     // ---------------- SEPMC tail (CTG:378-424, 458-470, 495-596, 640-652)
     const double* A = E.aux;
-    int counter = (int)A[env];
-    PS.with_flag = (int)A[N + env]; PS.flag_x = A[2 * N + env]; PS.flag_y = A[3 * N + env];
-    const float fix_spd = (float)A[4 * N + env];
-    double total_spd = A[7 * N + env], max_spd = A[8 * N + env];
-    PS.flag_draws = (int)A[15 * N + env];
+    int counter = (int)A[aux::counter * N + env];
+    PS.with_flag = (int)A[aux::with_flag * N + env]; PS.flag_x = A[aux::flag_x * N + env]; PS.flag_y = A[aux::flag_y * N + env];
+    const float fix_spd = (float)A[aux::control_spd * N + env];
+    double total_spd = A[aux::total_spd * N + env], max_spd = A[aux::max_spd * N + env];
+    PS.flag_draws = (int)A[aux::flag_draws * N + env];
     qb = qmul(qp, qI);
     float* snew = s_new + el * kNewObs;
     const float* spart = s_new + (el ^ 1) * kNewObs;
-    sepmc_pair_tail<4>(M, L, k, robot, snew, spart, px, py, pz, qp, qb, vw, ww, q, touch_own, fix_spd, seed, pair_gid, epi, PS);
+    sepmc_pair_tail(M, L, k, robot, snew, spart, px, py, pz, qp, qb, vw, ww, q, touch_own, fix_spd, seed, pair_gid, epi, PS);
 #pragma unroll
     for (int t = 0; t < 3; t++) { snew[3 * k + t] = q[t]; snew[12 + 3 * k + t] = qd[t]; snew[kPropDim + 3 * k + t] = act_src[3 * k + t]; }
     const float spd = sqrtf(vw.x * vw.x + vw.y * vw.y);              // stat_spd (CTG:368-373)
     total_spd += (double)spd;
     if ((double)spd > max_spd) max_spd = (double)spd;
     counter += 1;
-    const M3 Rq = qmat(qnormalize(qb));
-    const float left_z = Rq.a02 * Rq.a10 - Rq.a12 * Rq.a00;
-    int fall = (left_z > 0.70710678118654752f || left_z < -0.70710678118654752f || Rq.a22 < 0.5f) ? 1 : 0;
+    int fall = fallen(qmat(qnormalize(qb))) ? 1 : 0;
     const int fall_other = __shfl_xor_sync(FULL, fall, 4);
     if (robot == 1) fall = fall_other;                                  // only robot 0's fall ends the episode (CTG:462)
     bad = bad || __shfl_xor_sync(FULL, bad ? 1 : 0, 4) != 0;
@@ -542,49 +522,36 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
     if (done && tag) rew += (wf0 != 0) == (robot == 0) ? 1.f : -1.f;
     if (bad) rew = 0.f;
     rew_out = rew;
-    V3 fd;
-    {
-      V3 f = mul(qmat(qp), foot_in_base(L, q[0], q[1], q[2]));
-      fd = V3{(float)px + f.x, (float)py + f.y, (float)pz + f.z};
-    }
     if (wr) {
-      float* sw = E.st;
-#pragma unroll
-      for (int t = 0; t < 3; t++) { sw[(10 + 3 * k + t) * N + env] = q[t]; sw[(22 + 3 * k + t) * N + env] = qd[t]; }
-      E.foot_pos[(3 * k) * N + env] = fd.x; E.foot_pos[(3 * k + 1) * N + env] = fd.y; E.foot_pos[(3 * k + 2) * N + env] = fd.z;
+      const V3 f = mul(qmat(qp), foot_in_base(L, q[0], q[1], q[2]));
+      store_state(E, N, env, k, q, qd, V3{(float)px + f.x, (float)py + f.y, (float)pz + f.z}, px, py, pz, qb, vw, ww);
       if (k == 0) {
-        E.pos[env] = px; E.pos[N + env] = py; E.pos[2 * N + env] = pz;
-        sw[env] = qb.x; sw[N + env] = qb.y; sw[2 * N + env] = qb.z; sw[3 * N + env] = qb.w;
-        sw[4 * N + env] = vw.x; sw[5 * N + env] = vw.y; sw[6 * N + env] = vw.z;
-        sw[7 * N + env] = ww.x; sw[8 * N + env] = ww.y; sw[9 * N + env] = ww.z;
-        E.time[env] = time;
-        E.reward_sum[env] += rew;
-        E.episode_steps[env] += 1;
-        E.reward[env] = rew;
-        E.done[env] = done ? 1 : 0;
         double* Aw = E.aux;
-        Aw[env] = counter; Aw[N + env] = PS.with_flag; Aw[2 * N + env] = PS.flag_x; Aw[3 * N + env] = PS.flag_y; Aw[5 * N + env] = PS.visible;
-        Aw[6 * N + env] = PS.sw; Aw[7 * N + env] = total_spd; Aw[8 * N + env] = max_spd; Aw[9 * N + env] = push_count;
-        Aw[10 * N + env] = pf[0]; Aw[11 * N + env] = pf[1]; Aw[12 * N + env] = pf[2]; Aw[14 * N + env] = push_draws; Aw[15 * N + env] = PS.flag_draws;
-        Aw[17 * N + env] = touch_own ? 1.0 : 0.0;
+        Aw[aux::counter * N + env] = counter; Aw[aux::with_flag * N + env] = PS.with_flag; Aw[aux::flag_x * N + env] = PS.flag_x;
+        Aw[aux::flag_y * N + env] = PS.flag_y; Aw[aux::oppo_visible * N + env] = PS.visible; Aw[aux::switch_flag * N + env] = PS.sw;
+        Aw[aux::total_spd * N + env] = total_spd; Aw[aux::max_spd * N + env] = max_spd; Aw[aux::push_count * N + env] = push_count;
+        Aw[aux::push_fx * N + env] = pf[0]; Aw[aux::push_fy * N + env] = pf[1]; Aw[aux::push_fz * N + env] = pf[2];
+        Aw[aux::push_draws * N + env] = push_draws; Aw[aux::flag_draws * N + env] = PS.flag_draws;
+        Aw[aux::flag_touch * N + env] = touch_own ? 1.0 : 0.0;
       }
     }
   } else {
     // ---------------- EPMC tail (PGE:302-321, 334-358, 360-372, 479-539)
     const double* A = E.aux;
-    int counter = (int)A[env], cmd_draws = (int)A[15 * N + env];
-    const int cmd_freq = (int)A[N + env];
-    double tgx = A[2 * N + env], tgy = A[3 * N + env], target_angle = A[5 * N + env], last_len = A[6 * N + env];
-    double total_spd = A[7 * N + env], max_spd = A[8 * N + env];
-    float target_spd = (float)A[4 * N + env];
-    const double init_len = ENV == 3 ? A[17 * N + env] : 1.0;
+    int counter = (int)A[aux::counter * N + env], cmd_draws = (int)A[aux::cmd_draws * N + env];
+    const int cmd_freq = (int)A[aux::cmd_vary_freq * N + env];
+    double tgx = A[aux::target_x * N + env], tgy = A[aux::target_y * N + env], target_angle = A[aux::target_angle * N + env];
+    double last_len = A[aux::last_pos_diff_len * N + env];
+    double total_spd = A[aux::total_spd * N + env], max_spd = A[aux::max_spd * N + env];
+    float target_spd = (float)A[aux::target_spd * N + env];
+    const double init_len = ENV == kEpmcCorridor ? A[aux::init_pos_diff_len * N + env] : 1.0;
     {
       // the command of this step was drawn from the pose at the START of the step (PGE:302-317): recover it from the stored state
       const double sx0 = E.pos[env], sy0 = E.pos[N + env];
       if (counter % cmd_freq == 0) {
         double uu[4];
         stream_uniforms(seed, gid0 + env, epi, 3, (unsigned)cmd_draws++, uu);
-        if (ENV == 1) {
+        if (ENV == kEpmcFlat) {
           target_angle = 2.0 * 3.14159265358979323846 * uu[0];
           double sn, cs;
           sincos(target_angle, &sn, &cs);
@@ -593,7 +560,7 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
         }
         target_spd = (float)((double)P.ts_lo + uu[1] * ((double)P.ts_hi - (double)P.ts_lo));
       }
-      if (ENV == 3) target_angle = atan2(tgy - sy0, tgx - sx0);            // PGE:318-323 (plotting only)
+      if (ENV == kEpmcCorridor) target_angle = atan2(tgy - sy0, tgx - sx0);     // PGE:318-323 (plotting only)
     }
     __syncwarp();                                        // the pose above is read before lane 0 overwrites it below
     qb = qmul(qp, qI);
@@ -605,20 +572,8 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
     counter += 1;
     const double dx = tgx - px, dy = tgy - py;
     const double plen = sqrt(dx * dx + dy * dy);
-    if (k == 0) {
-      V3 wl = tmul(Rq, ww), vl = tmul(Rq, vw);
-      snew[24] = wl.x; snew[25] = wl.y; snew[26] = wl.z; snew[27] = vl.x; snew[28] = vl.y; snew[29] = vl.z;
-      snew[30] = Rq.a20; snew[31] = Rq.a21; snew[32] = Rq.a22;
-      snew[45] = Rq.a00; snew[46] = Rq.a01; snew[47] = Rq.a02; snew[48] = Rq.a10; snew[49] = Rq.a11; snew[50] = Rq.a12;
-      snew[51] = Rq.a20; snew[52] = Rq.a21; snew[53] = Rq.a22;
-      snew[54] = (float)px; snew[55] = (float)py; snew[56] = (float)pz;
-      V3 dd = tmul(Rq, V3{(float)dx, (float)dy, (float)(0.0 - pz)});
-      float n2_ = sqrtf(dd.x * dd.x + dd.y * dd.y);
-      snew[57] = dd.x / n2_; snew[58] = dd.y / n2_; snew[59] = target_spd;
-      snew[60] = (float)sqrt(px * px + py * py + pz * pz);
-    }
-    const float left_z = Rq.a02 * Rq.a10 - Rq.a12 * Rq.a00;
-    const bool fall = left_z > 0.70710678118654752f || left_z < -0.70710678118654752f || Rq.a22 < 0.5f;
+    if (k == 0) stage_epmc(snew, Rq, ww, vw, px, py, pz, dx, dy, target_spd);
+    const bool fall = fallen(Rq);
     const bool reach = plen < 0.5, timeup = counter >= P.max_steps;
     const float ux = (float)(dx / plen), uy = (float)(dy / plen);
     const float spd = fabsf(vw.x * ux + vw.y * uy);
@@ -628,7 +583,7 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
     float sy_, cy_;
     llq_sincosf(yaw, &sy_, &cy_);
     float rew = expf(-fabsf(spd - target_spd)) * expf((cy_ * ux + sy_ * uy - 1.0f) * 5.0f) / (float)P.max_steps;
-    if (ENV == 3) {                                                    // _compute_avg_spd_reward (PGE:504-539)
+    if (ENV == kEpmcCorridor) {                                        // _compute_avg_spd_reward (PGE:504-539)
       const float reward_rot = expf((cy_ * ux + sy_ * uy - 1.0f) * 5.0f);
       const float reward_dist = (float)((plen - last_len) / init_len);
       last_len = plen;
@@ -639,33 +594,26 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
     if (bad || !isfinite(rew)) { rew = 0.f; bad = true; }
     done = fall || timeup || reach || bad;
     rew_out = rew;
-    V3 fd;
-    {
-      V3 f = mul(qmat(qp), foot_in_base(L, q[0], q[1], q[2]));
-      fd = V3{(float)px + f.x, (float)py + f.y, (float)pz + f.z};
-    }
     if (wr) {
-      float* sw = E.st;
-#pragma unroll
-      for (int t = 0; t < 3; t++) { sw[(10 + 3 * k + t) * N + env] = q[t]; sw[(22 + 3 * k + t) * N + env] = qd[t]; }
-      E.foot_pos[(3 * k) * N + env] = fd.x; E.foot_pos[(3 * k + 1) * N + env] = fd.y; E.foot_pos[(3 * k + 2) * N + env] = fd.z;
+      const V3 f = mul(qmat(qp), foot_in_base(L, q[0], q[1], q[2]));
+      store_state(E, N, env, k, q, qd, V3{(float)px + f.x, (float)py + f.y, (float)pz + f.z}, px, py, pz, qb, vw, ww);
       if (k == 0) {
-        E.pos[env] = px; E.pos[N + env] = py; E.pos[2 * N + env] = pz;
-        sw[env] = qb.x; sw[N + env] = qb.y; sw[2 * N + env] = qb.z; sw[3 * N + env] = qb.w;
-        sw[4 * N + env] = vw.x; sw[5 * N + env] = vw.y; sw[6 * N + env] = vw.z;
-        sw[7 * N + env] = ww.x; sw[8 * N + env] = ww.y; sw[9 * N + env] = ww.z;
-        E.time[env] = time;
-        E.reward_sum[env] += rew;
-        E.episode_steps[env] += 1;
-        E.reward[env] = rew;
-        E.done[env] = done ? 1 : 0;
         double* Aw = E.aux;
-        Aw[env] = counter; Aw[N + env] = cmd_freq; Aw[2 * N + env] = tgx; Aw[3 * N + env] = tgy; Aw[4 * N + env] = target_spd;
-        Aw[5 * N + env] = target_angle; Aw[6 * N + env] = last_len; Aw[7 * N + env] = total_spd; Aw[8 * N + env] = max_spd;
-        Aw[9 * N + env] = push_count; Aw[10 * N + env] = pf[0]; Aw[11 * N + env] = pf[1]; Aw[12 * N + env] = pf[2];
-        Aw[14 * N + env] = push_draws; Aw[15 * N + env] = cmd_draws;
+        Aw[aux::counter * N + env] = counter; Aw[aux::cmd_vary_freq * N + env] = cmd_freq; Aw[aux::target_x * N + env] = tgx;
+        Aw[aux::target_y * N + env] = tgy; Aw[aux::target_spd * N + env] = target_spd; Aw[aux::target_angle * N + env] = target_angle;
+        Aw[aux::last_pos_diff_len * N + env] = last_len; Aw[aux::total_spd * N + env] = total_spd; Aw[aux::max_spd * N + env] = max_spd;
+        Aw[aux::push_count * N + env] = push_count;
+        Aw[aux::push_fx * N + env] = pf[0]; Aw[aux::push_fy * N + env] = pf[1]; Aw[aux::push_fz * N + env] = pf[2];
+        Aw[aux::push_draws * N + env] = push_draws; Aw[aux::cmd_draws * N + env] = cmd_draws;
       }
     }
+  }
+  if (wr && k == 0) {                                    // end-of-step bookkeeping of every level
+    E.time[env] = time;
+    E.reward_sum[env] += rew_out;
+    E.episode_steps[env] += 1;
+    E.reward[env] = rew_out;
+    E.done[env] = done ? 1 : 0;
   }
   // record mode (llq_set_option "record"): the trajectory columns action 12 | reward | done behind the observation of the slab row;
   // record == 2: into the slab row before the one that receives the observation (parallel/rollout.py)
@@ -754,10 +702,10 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
   warm[0] = l16 < nsph ? E.warm[(size_t)l16 * N + env] : 0.f;
   warm[1] = 16 + l16 < nsph ? E.warm[(size_t)(16 + l16) * N + env] : 0.f;
   double time = E.time[env];
-  const int clip = ENV == 0 ? E.clip[env] : 0;
+  const int clip = ENV == kPmc ? E.clip[env] : 0;
   int frame_id = 0; double frame_frac = 0.0;
   int ob_id = 0; bool ob_hit = false;
-  if (ENV == 0 && P.has_ob) ob_id = E.ob_id[env];
+  if (ENV == kPmc && P.has_ob) ob_id = E.ob_id[env];
   // ---- EPMC / SEPMC bookkeeping used inside the sub-steps (the rest is read in the tail)
   int push_count = 0, push_draws = 0;
   float pf[3] = {0.f, 0.f, 0.f}, mu_env = P.mu;
@@ -766,18 +714,18 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
   bool touch_own = false, tag = false;
   const int robot = env & 1;
   const long long pair_gid = gid0 + (env & ~1);
-  if (ENV != 0) {
+  if (ENV != kPmc) {
     const double* A = E.aux;
-    push_count = (int)A[9 * N + env];
-    pf[0] = (float)A[10 * N + env]; pf[1] = (float)A[11 * N + env]; pf[2] = (float)A[12 * N + env];
-    mu_env = P.mu_ground * (float)A[13 * N + env]; push_draws = (int)A[14 * N + env];
+    push_count = (int)A[aux::push_count * N + env];
+    pf[0] = (float)A[aux::push_fx * N + env]; pf[1] = (float)A[aux::push_fy * N + env]; pf[2] = (float)A[aux::push_fz * N + env];
+    mu_env = P.mu_ground * (float)A[aux::foot_friction * N + env]; push_draws = (int)A[aux::push_draws * N + env];
     epi = E.episode[env] - 1;                             // streams of the running episode (the reset advanced the counter)
-    if (ENV == 2) { PS.flag_x = A[2 * N + env]; PS.flag_y = A[3 * N + env]; }
+    if (ENV == kSepmc) { PS.flag_x = A[aux::flag_x * N + env]; PS.flag_y = A[aux::flag_y * N + env]; }
   }
   // ---- EPMC corridor: the boxes the robot can reach during this step -> shared memory (<= kMaxCand per env)
   int n_cand = 0;
   float* s_cand = nullptr;
-  if (ENV == 3) {
+  if (ENV == kEpmcCorridor) {
     s_cand = &s_new[el][0];                            // the staging row is free until the tail: 8 x 6 floats
     const float* bxs = E.boxes + (size_t)env * (6 * kMaxBoxes);
     // reach of the robot's spheres from the base reference point: hip offset 0.195 + leg 0.48 in x, 0.15 + 0.05 in y, plus the
@@ -801,7 +749,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
   Q4 qp = qmul(qnormalize(qb), qconj(qI));
   unsigned n_contact_rows = 0, n_limit_rows = 0, n_overflow = 0;
   bool bad = false;
-  const float mu_foot = ENV != 0 ? mu_env : P.mu;
+  const float mu_foot = ENV != kPmc ? mu_env : P.mu;
 
   T16_DECL;
   for (int sub = 0; sub < P.substeps; sub++) {
@@ -809,18 +757,19 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     const float dt = P.dt;
     // ---------------- push randomiser (PR:56-87): counters in sub-steps, force lasts one sub-step
     bool push_on = false;
-    if (ENV == 2 && P.push_enabled) {
+    if (ENV == kSepmc && P.push_enabled) {
       push_count += 1;
       if (push_count > 0) {
         if (push_count % P.push_interval == 0) { push_draws += 1; push_count = 0; }
         if (push_count < P.push_duration) {
-          push_force_of_draw(P, seed, pair_gid, epi, push_draws - 1 + robot, pf);
+          int draw = push_draws - 1 + robot;
+          epmc_randomize_push(P, seed, pair_gid, epi, draw, pf);
           push_draws += 2;
           push_on = true;
         }
       }
     }
-    if ((ENV == 1 || ENV == 3) && P.push_enabled) {
+    if ((ENV == kEpmcFlat || ENV == kEpmcCorridor) && P.push_enabled) {
       push_count += 1;
       if (push_count > 0) {
         if (push_count % P.push_interval == 0) { epmc_randomize_push(P, seed, gid0 + env, epi, push_draws, pf); push_count = 0; }
@@ -879,7 +828,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     SV f = bias_wrench(bm_, hc, Ic, nd, dp, v.a, v.l, P.kl, P.ka, cy, sy, cx, sx, po);
     f.a = f.a + mul(Ic, ab.a) + cross(hc, ab.l);
     f.l = f.l + bm_ * ab.l + cross(ab.a, hc);
-    if (ENV != 0 && push_on && l16 == 0) {
+    if (ENV != kPmc && push_on && l16 == 0) {
       // applyExternalForce(link 0 = FR hip, LINK_FRAME): force given in the hip's inertial frame, applied at its CoM (PR:73-77)
       const V3 fl = V3{M.push_R[0] * pf[0] + M.push_R[1] * pf[1] + M.push_R[2] * pf[2], M.push_R[3] * pf[0] + M.push_R[4] * pf[1] + M.push_R[5] * pf[2],
                        M.push_R[6] * pf[0] + M.push_R[7] * pf[1] + M.push_R[8] * pf[2]};
@@ -1040,7 +989,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     __syncwarp();
     const M3 R = qmat(qp);                            // world <- B' (recomputed: cheaper than keeping nine registers alive)
     // ---------------- PMC hurdle plate: getContactPoints (PLE:343) reports the manifolds built on the last sub-step's pre-step poses
-    if (ENV == 0 && P.has_ob && sub == P.substeps - 1) {
+    if (ENV == kPmc && P.has_ob && sub == P.substeps - 1) {
       const int o0 = mc.ob_off[clip], n_ob = mc.ob_off[clip + 1] - o0;
       if (n_ob > 0) {
         const float* lk = linktab + 24 * k;
@@ -1061,7 +1010,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
       }
     }
     // ---------------- SEPMC: getContactPoints() (CTG:426-456) = manifolds of the last sub-step, built on its pre-step poses
-    if (ENV == 2 && sub == P.substeps - 1) {
+    if (ENV == kSepmc && sub == P.substeps - 1) {
       float* srow = &s_new[el][0];
       const float* prow = &s_new[el ^ 1][0];
       const V3 pw = V3{(float)px, (float)py, (float)pz};
@@ -1129,12 +1078,12 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
         float dist = (float)pz + dot(nb, cb) - sp.r;                // fp32 screen
         const bool statics = rule == 2 || s < 4;                    // legacy rules: only the feet touch walls and boxes
         bool near_ = have && dist < P.breaking + 0.01f;
-        if (ENV == 2 && statics && have) {
+        if (ENV == kSepmc && statics && have) {
           const V3 cw = V3{(float)px, (float)py, (float)pz} + mul(R, cb);
           near_ = near_ || fmaxf(fabsf(cw.x), fabsf(cw.y)) + sp.r > kWallIn - P.breaking - 0.01f;
         }
-        unsigned cmask = 0;                              // ENV 3: candidate boxes this sphere can touch (fp32 screen, 3 cm of slack)
-        if (ENV == 3 && statics && have && n_cand > 0) {
+        unsigned cmask = 0;                              // EPMC corridor: candidate boxes this sphere can touch (fp32 screen, 3 cm of slack)
+        if (ENV == kEpmcCorridor && statics && have && n_cand > 0) {
           const V3 cw = V3{(float)px, (float)py, (float)pz} + mul(R, cb);
           const float reach = sp.r + P.aux_r + P.breaking + 0.03f;
           for (int c = 0; c < n_cand; c++) {
@@ -1168,10 +1117,10 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
               x += (double)SL.j[0].r[0]; y += (double)SL.j[0].r[1]; z += (double)SL.j[0].r[2];
             }
             dist = (float)(pz + nx * x + ny * y + nz * z - (double)sp.r);
-            if ((ENV == 2 || ENV == 3) && statics) {
+            if ((ENV == kSepmc || ENV == kEpmcCorridor) && statics) {
               const double wx = px + (1.0 - 2.0 * (qy * qy + qz * qz)) * x + 2.0 * (qx * qy - qz * qw) * y + 2.0 * (qx * qz + qy * qw) * z;
               const double wy = py + 2.0 * (qx * qy + qz * qw) * x + (1.0 - 2.0 * (qx * qx + qz * qz)) * y + 2.0 * (qy * qz - qx * qw) * z;
-              if (ENV == 2) {
+              if (ENV == kSepmc) {
                 // the arena walls (BSG:863-902) as four more half-spaces; one contact per sphere, the deepest (DESIGN.md 5)
                 const double lim = (double)kWallIn - (double)sp.r;
                 const float d1 = (float)(lim - wx), d2 = (float)(lim + wx), d3 = (float)(lim - wy), d4 = (float)(lim + wy);
@@ -1220,7 +1169,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
         if (contact) {
           // directions (base coordinates): normal, then btPlaneSpace1's two tangents
           V3 dn = nb, d1_ = neg(V3{R.a10, R.a11, R.a12}), d2_ = V3{R.a00, R.a01, R.a02};   // ground: n = +z, t1 = -y, t2 = +x (world)
-          if (ENV == 2 && plane != 0) {
+          if (ENV == kSepmc && plane != 0) {
             const V3 w0 = V3{R.a00, R.a01, R.a02}, w1 = V3{R.a10, R.a11, R.a12};
             d2_ = nb;                                     // t2 = +z for every wall
             if (plane == 1) { dn = neg(w0); d1_ = neg(w1); }
@@ -1228,7 +1177,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
             else if (plane == 3) { dn = neg(w1); d1_ = w0; }
             else { dn = w1; d1_ = neg(w0); }
           }
-          if (ENV == 3 && plane == 5) {                   // general normal: btPlaneSpace1 in world axes, then into base coordinates
+          if (ENV == kEpmcCorridor && plane == 5) {                   // general normal: btPlaneSpace1 in world axes, then into base coordinates
             const V3 n = nworld;
             V3 t1, t2;
             if (fabsf(n.z) > 0.70710678118654752f) {
@@ -1375,7 +1324,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     }
     bad = bad || !(fabsf(qd[0]) <= P.vmax) || !(fabsf(ww.x) <= P.vmax) || !(fabsf(vw.x) <= P.vmax);
     // ---------------- mocap clock (PLE:208-210): sampled with the time *before* the increment
-    if (ENV == 0 && sub == P.substeps - 1) {
+    if (ENV == kPmc && sub == P.substeps - 1) {
       frame_id = (int)floor(time / P.frame_dt);
       frame_frac = (time - frame_id * P.frame_dt) / P.frame_dt;
       const int last = mc.clip_off[clip + 1] - mc.clip_off[clip] - P.margin + 2;     // see llq_kernels.cuh: runaway cursors only
