@@ -20,6 +20,8 @@
 #include <string>
 #include <vector>
 
+static_assert(llq::state::dim == LLQ_STATE_DIM && llq::kRecW == LLQ_ACTION_DIM + 2, "state and record layouts of include/llq.h");
+
 namespace {
 
 thread_local std::string g_err;
@@ -251,9 +253,9 @@ int llq_create(const llq_config* cfg, llq_handle* out) {
   cudaError_t ce = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
   if (ce != cudaSuccess) { delete h; return fail(LLQ_ECUDA, cudaGetErrorString(ce)); }
   TRY(dalloc(&h->d_model, 1)); TRY(dalloc(&h->d_sph, 1));
-  TRY(dalloc(&h->E.pos, 3 * n)); TRY(dalloc(&h->E.st, 34 * n)); TRY(dalloc(&h->E.time, n)); TRY(dalloc(&h->E.clip, n));
+  TRY(dalloc(&h->E.pos, 3 * n)); TRY(dalloc(&h->E.st, llq::st::dim * n)); TRY(dalloc(&h->E.time, n)); TRY(dalloc(&h->E.clip, n));
   TRY(dalloc(&h->E.reward_sum, n)); TRY(dalloc(&h->E.episode_steps, n)); TRY(dalloc(&h->E.episode, n));
-  TRY(dalloc(&h->E.warm, LLQ_MAX_SPHERES * n)); TRY(dalloc(&h->E.obs, (size_t)h->obs_dim * n)); TRY(dalloc(&h->E.kin, 37 * n));
+  TRY(dalloc(&h->E.warm, LLQ_MAX_SPHERES * n)); TRY(dalloc(&h->E.obs, (size_t)h->obs_dim * n)); TRY(dalloc(&h->E.kin, llq::state::dim * n));
   TRY(dalloc(&h->E.foot_pos, 12 * n)); TRY(dalloc(&h->E.done_reward, n)); TRY(dalloc(&h->E.done, n)); TRY(dalloc(&h->E.reward, n));
   TRY(dalloc(&h->E.counters, 8));
   TRY(dalloc(&h->E.aux, (size_t)LLQ_AUX_DIM * n));
@@ -395,7 +397,7 @@ int llq_load_model(llq_handle h, const double* b, int64_t n) {
     if (nfoot != 4) return fail(LLQ_EINVAL, "model blob must list the four foot spheres first");
     CK(cudaMemcpy(h->d_sph, &T, sizeof(T), cudaMemcpyHostToDevice));
   }
-  for (int i = 0; i < 37; i++) M.init_state[i] = h->h_model.init_state[i];
+  for (int i = 0; i < llq::state::dim; i++) M.init_state[i] = h->h_model.init_state[i];
   h->h_model = M;
   CK(cudaMemcpy(h->d_model, &M, sizeof(M), cudaMemcpyHostToDevice));
   h->has_model = true;
@@ -408,7 +410,7 @@ int llq_set_init_state(llq_handle h, const double* st) {
   if (!h || !st) return fail(LLQ_EINVAL, "null argument");
   int rc = set_device(h);
   if (rc) return rc;
-  for (int i = 0; i < 37; i++) h->h_model.init_state[i] = (float)st[i];
+  for (int i = 0; i < llq::state::dim; i++) h->h_model.init_state[i] = (float)st[i];
   if (h->has_model) CK(cudaMemcpy(h->d_model, &h->h_model, sizeof(h->h_model), cudaMemcpyHostToDevice));
   h->has_init_state = true;
   return LLQ_OK;
@@ -533,8 +535,8 @@ int llq_step_ex(llq_handle h, const float* actions, float* obs, int64_t obs_ld, 
   if (!actions) return fail(LLQ_EINVAL, "null actions");
   const size_t od = (size_t)h->obs_dim;
   if (obs && obs_ld < (int64_t)od) return fail(LLQ_EINVAL, "obs_ld smaller than the observation width");
-  if (h->record && io_mode == LLQ_IO_DEVICE && obs && obs_ld < (int64_t)od + 14)
-    return fail(LLQ_EINVAL, "record mode needs obs_ld >= observation width + 14 (action 12 | reward | done)");
+  if (h->record && io_mode == LLQ_IO_DEVICE && obs && obs_ld < (int64_t)od + llq::kRecW)
+    return fail(LLQ_EINVAL, "record mode needs obs_ld >= observation width + " + std::to_string(llq::kRecW) + " (action | reward | done)");
   const size_t n = (size_t)h->cfg.n_envs;
   llq::EnvArrays E = h->E;
   const float* d_act;
@@ -603,19 +605,19 @@ int llq_get_field(llq_handle h, int field, void* dst) {
   CK(cudaStreamSynchronize(h->stream));
   switch (field) {
     case LLQ_F_STATE: {
-      std::vector<float> tmp(34 * n);
-      rc = get_soa_f(h, h->E.st, 34, tmp.data());
+      std::vector<float> tmp(llq::st::dim * n);
+      rc = get_soa_f(h, h->E.st, llq::st::dim, tmp.data());
       if (rc) return rc;
       std::vector<double> pos(3 * n);
       CK(cudaMemcpy(pos.data(), h->E.pos, sizeof(double) * 3 * n, cudaMemcpyDeviceToHost));
       float* o = (float*)dst;
       for (size_t i = 0; i < n; i++) {
-        for (int t = 0; t < 3; t++) o[i * 37 + t] = (float)pos[t * n + i];
-        for (int t = 0; t < 34; t++) o[i * 37 + 3 + t] = tmp[i * 34 + t];
+        for (int t = 0; t < 3; t++) o[i * llq::state::dim + llq::state::pos + t] = (float)pos[t * n + i];
+        for (int t = 0; t < llq::st::dim; t++) o[i * llq::state::dim + llq::state::quat + t] = tmp[i * llq::st::dim + t];
       }
       return LLQ_OK;
     }
-    case LLQ_F_KIN_STATE: return get_soa_f(h, h->E.kin, 37, (float*)dst);
+    case LLQ_F_KIN_STATE: return get_soa_f(h, h->E.kin, llq::state::dim, (float*)dst);
     case LLQ_F_WARMSTART: return get_soa_f(h, h->E.warm, LLQ_MAX_SPHERES, (float*)dst);
     case LLQ_F_FOOT_POS: return get_soa_f(h, h->E.foot_pos, 12, (float*)dst);
     case LLQ_F_CLIP: CK(cudaMemcpy(dst, h->E.clip, sizeof(int) * n, cudaMemcpyDeviceToHost)); return LLQ_OK;
@@ -661,12 +663,12 @@ int llq_set_field(llq_handle h, int field, const void* src) {
   switch (field) {
     case LLQ_F_STATE: {
       const float* s = (const float*)src;
-      std::vector<float> st(34 * n); std::vector<double> pos(3 * n);
+      std::vector<float> st(llq::st::dim * n); std::vector<double> pos(3 * n);
       for (size_t i = 0; i < n; i++) {
-        for (int t = 0; t < 3; t++) pos[t * n + i] = (double)s[i * 37 + t];
-        for (int t = 0; t < 34; t++) st[t * n + i] = s[i * 37 + 3 + t];
+        for (int t = 0; t < 3; t++) pos[t * n + i] = (double)s[i * llq::state::dim + llq::state::pos + t];
+        for (int t = 0; t < llq::st::dim; t++) st[t * n + i] = s[i * llq::state::dim + llq::state::quat + t];
       }
-      CK(cudaMemcpy(h->E.st, st.data(), sizeof(float) * 34 * n, cudaMemcpyHostToDevice));
+      CK(cudaMemcpy(h->E.st, st.data(), sizeof(float) * llq::st::dim * n, cudaMemcpyHostToDevice));
       CK(cudaMemcpy(h->E.pos, pos.data(), sizeof(double) * 3 * n, cudaMemcpyHostToDevice));
       return LLQ_OK;
     }

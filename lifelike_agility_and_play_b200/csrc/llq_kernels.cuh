@@ -41,6 +41,16 @@ constexpr int counter = 0, cmd_vary_freq = 1, target_x = 2, target_y = 3, target
               cmd_draws = 15, yaw_accum_deg = 16, init_pos_diff_len = 17;
 constexpr int with_flag = 1, flag_x = 2, flag_y = 3, control_spd = 4, oppo_visible = 5, switch_flag = 6, flag_draws = 15, flag_touch = 17;
 }  // namespace aux
+// rows of the robot state (pybullet base-inertial convention, LR:86-106): LLQ_F_STATE, E.kin and M.init_state use all 37
+namespace state {
+constexpr int pos = 0, quat = 3, lin = 7, ang = 10, q = 13, qd = 25, dim = 37;
+}  // namespace state
+// rows of E.st: the same layout without pos, which E.pos keeps in fp64
+namespace st {
+constexpr int quat = state::quat - 3, lin = state::lin - 3, ang = state::ang - 3, q = state::q - 3, qd = state::qd - 3, dim = state::dim - 3;
+}  // namespace st
+// record mode: the trajectory columns behind the observation of a slab row, action 12 | reward | done
+constexpr int kRecReward = kActDim, kRecDone = kActDim + 1, kRecW = kActDim + 2;
 
 struct DampItem { float m; float c[3]; float Ic[6]; };
 struct JointConst {
@@ -54,7 +64,7 @@ struct BaseConst { float qI[4]; float m; float h[3]; float I[6]; int nd; DampIte
 struct alignas(16) ModelConst {
   BaseConst base; LegConst leg[4];
   float push_R[9]; float push_c[3];   // FR hip link: inertial-frame rotation (link <- inertial) and CoM, for applyExternalForce(LINK_FRAME) (PR:73-77)
-  float init_state[37]; float pad_[3]; // EPMC episode start state (LR:115-117, utils/constants.py:103-116)
+  float init_state[state::dim]; float pad_[3]; // EPMC episode start state (LR:115-117, utils/constants.py:103-116)
   // detection proxies for the PMC hurdle plate: wheel (knee) centre in the thigh frame + radius, hip radius, body-box corners (base coords)
   float wheel_off[4][3]; float wheel_r[4]; float hip_r[4]; float corner[8][3];
   float handle[2][4];                  // SEPMC: front / hind handle centre (base coords) + radius (LR:150-156)
@@ -82,7 +92,7 @@ struct StepParams {
 
 struct EnvArrays {      // SoA device arrays, N envs
   double* pos;          // [3][N]
-  float* st;            // [34][N]: quat4 lin3 ang3 q12 qd12
+  float* st;            // [34][N]: rows st::
   double* time;         // [N]
   int* clip;            // [N]
   float* reward_sum;    // [N]
@@ -90,7 +100,7 @@ struct EnvArrays {      // SoA device arrays, N envs
   long long* episode;   // [N]
   float* warm;          // [4][N]
   float* obs;           // [N][207] (history carry)
-  float* kin;           // [37][N]
+  float* kin;           // [37][N]: rows state::
   float* foot_pos;      // [12][N]
   float* done_reward;   // [N] reward_sum at termination
   unsigned char* done;  // [N]
@@ -193,15 +203,17 @@ LLQ_DI void store_state(const EnvArrays& E, int N, int env, int k, const float (
                         double pz, Q4 qb, V3 lin, V3 ang) {
   float* sw = E.st;
 #pragma unroll
-  for (int t = 0; t < 3; t++) { sw[(10 + 3 * k + t) * N + env] = q[t]; sw[(22 + 3 * k + t) * N + env] = qd[t]; }
+  for (int t = 0; t < 3; t++) { sw[(st::q + 3 * k + t) * N + env] = q[t]; sw[(st::qd + 3 * k + t) * N + env] = qd[t]; }
   E.foot_pos[(3 * k) * N + env] = foot.x; E.foot_pos[(3 * k + 1) * N + env] = foot.y; E.foot_pos[(3 * k + 2) * N + env] = foot.z;
   if (k == 0) {
     E.pos[env] = px; E.pos[N + env] = py; E.pos[2 * N + env] = pz;
-    sw[env] = qb.x; sw[N + env] = qb.y; sw[2 * N + env] = qb.z; sw[3 * N + env] = qb.w;
-    sw[4 * N + env] = lin.x; sw[5 * N + env] = lin.y; sw[6 * N + env] = lin.z;
-    sw[7 * N + env] = ang.x; sw[8 * N + env] = ang.y; sw[9 * N + env] = ang.z;
+    sw[st::quat * N + env] = qb.x; sw[(st::quat + 1) * N + env] = qb.y; sw[(st::quat + 2) * N + env] = qb.z; sw[(st::quat + 3) * N + env] = qb.w;
+    sw[st::lin * N + env] = lin.x; sw[(st::lin + 1) * N + env] = lin.y; sw[(st::lin + 2) * N + env] = lin.z;
+    sw[st::ang * N + env] = ang.x; sw[(st::ang + 1) * N + env] = ang.y; sw[(st::ang + 2) * N + env] = ang.z;
   }
 }
+// rotation of the base's inertial frame (pybullet's base orientation) in the URDF body axes: q_inertial = q_body qI
+LLQ_DI Q4 base_qI(const ModelConst& M) { return Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]}; }
 // EPMC / SEPMC episode start (LR:115-117): M.init_state with the base yawed by yaw_deg about world z, this leg's joints.  The
 // outputs are references, not one returned struct: with the struct, nvcc 12.9 contracts a product of the reset's foot rotation
 // into a different FMA, and the reset foot positions change in the last bit.
@@ -210,9 +222,10 @@ LLQ_DI Q4 start_pose(const ModelConst& M, int k, double yaw_deg, float (&q)[3], 
   sincos(0.5 * yaw_deg * (3.14159265358979323846 / 180.0), &sn, &cs);
   const float* I0 = M.init_state;
 #pragma unroll
-  for (int i = 0; i < 3; i++) { q[i] = I0[13 + 3 * k + i]; qd[i] = I0[25 + 3 * k + i]; }
-  lin = V3{I0[7], I0[8], I0[9]}; ang = V3{I0[10], I0[11], I0[12]};
-  return qmul(qnormalize(Q4{I0[3], I0[4], I0[5], I0[6]}), Q4{0.f, 0.f, (float)sn, (float)cs});
+  for (int i = 0; i < 3; i++) { q[i] = I0[state::q + 3 * k + i]; qd[i] = I0[state::qd + 3 * k + i]; }
+  lin = ld3(I0 + state::lin); ang = ld3(I0 + state::ang);
+  const Q4 q0 = Q4{I0[state::quat], I0[state::quat + 1], I0[state::quat + 2], I0[state::quat + 3]};
+  return qmul(qnormalize(q0), Q4{0.f, 0.f, (float)sn, (float)cs});
 }
 // termination on the base orientation (LR:158-179), R = world <- base inertial
 LLQ_DI bool fallen(const M3& R) {
@@ -831,7 +844,7 @@ __global__ void __launch_bounds__(BLOCK) pmc_reset_kernel(EnvArrays E, MocapDev 
     float q[3], qd[3];
     V3 lin, ang;
     const Q4 qn = start_pose(M, k, robot == 0 ? yaw_a : yaw_b, q, qd, lin, ang);
-    const Q4 qI = Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]};
+    const Q4 qI = base_qI(M);
     const Q4 qp = qmul(qnormalize(qn), qconj(qI));
     PairState PS = {robot == 0 ? wflag : 1 - wflag, 0, 1, 0, -2.0 + 4.0 * u2[1], -2.0 + 4.0 * u2[2]};
     // reset() runs _prepare_drill too (CTG:302): its flag-switch test reads the stale manifolds of the previous episode's last step
@@ -890,7 +903,7 @@ __global__ void __launch_bounds__(BLOCK) pmc_reset_kernel(EnvArrays E, MocapDev 
       stage_corridor_masks(snew, E.boxes + (size_t)env * (6 * kMaxBoxes), doit ? nb0 : E.nbox[env], k, 0.f, 0.f, 0.5f, atan2f(Rq.a10, Rq.a00));
     }
     if (doit) {
-      const Q4 qI = Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]};
+      const Q4 qI = base_qI(M);
       const V3 f = mul(qmat(qmul(qnormalize(qn), qconj(qI))), foot_in_base(L, q[0], q[1], q[2]));
       E.warm[k * N + env] = 0.f;
       store_state(E, N, env, k, q, qd, V3{f.x, f.y, 0.5f + f.z}, 0.0, 0.0, 0.5, qn, lin, ang);
@@ -944,17 +957,17 @@ __global__ void __launch_bounds__(BLOCK) pmc_reset_kernel(EnvArrays E, MocapDev 
   float* snew = &s_new[threadIdx.x >> 2][0];
   build_obs_new(mc, P, M, k, clip, frame_id, frac, kb.px, kb.py, kb.pz, kb.q, kb.lin, kb.ang, q, qd, snew);
   if (doit) {
-    const Q4 qI = Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]};
+    const Q4 qI = base_qI(M);
     const V3 f = mul(qmat(qmul(qnormalize(kb.q), qconj(qI))), foot_in_base(L, q[0], q[1], q[2]));
     store_state(E, N, env, k, q, qd, V3{(float)kb.px + f.x, (float)kb.py + f.y, (float)kb.pz + f.z}, kb.px, kb.py, kb.pz, kb.q, kb.lin, kb.ang);
 #pragma unroll
-    for (int i = 0; i < 3; i++) { E.kin[(13 + 3 * k + i) * N + env] = q[i]; E.kin[(25 + 3 * k + i) * N + env] = qd[i]; }
+    for (int i = 0; i < 3; i++) { E.kin[(state::q + 3 * k + i) * N + env] = q[i]; E.kin[(state::qd + 3 * k + i) * N + env] = qd[i]; }
     E.warm[k * N + env] = 0.f;
     if (k == 0) {
-      const float b[10] = {kb.q.x, kb.q.y, kb.q.z, kb.q.w, kb.lin.x, kb.lin.y, kb.lin.z, kb.ang.x, kb.ang.y, kb.ang.z};
-      E.kin[env] = (float)kb.px; E.kin[N + env] = (float)kb.py; E.kin[2 * N + env] = (float)kb.pz;
+      const float b[10] = {kb.q.x, kb.q.y, kb.q.z, kb.q.w, kb.lin.x, kb.lin.y, kb.lin.z, kb.ang.x, kb.ang.y, kb.ang.z};   // quat | lin | ang
+      E.kin[state::pos * N + env] = (float)kb.px; E.kin[(state::pos + 1) * N + env] = (float)kb.py; E.kin[(state::pos + 2) * N + env] = (float)kb.pz;
 #pragma unroll
-      for (int i = 0; i < 10; i++) E.kin[(3 + i) * N + env] = b[i];
+      for (int i = 0; i < 10; i++) E.kin[(state::quat + i) * N + env] = b[i];
       E.time[env] = t0; E.clip[env] = clip; E.reward_sum[env] = 0.f; E.episode_steps[env] = 0; E.episode[env] = ep;
       E.ob_id[env] = 0;                                            // PLE:179
     }

@@ -34,16 +34,64 @@ constexpr int kMaxSph = 32, kMaxCon = 8, kMaxLim = 8;
 struct SphConst { float c[3]; float r; float mu_link; int leg; int depth; int foot; };   // centre in the frame of link (leg, depth - 1); depth 0 = base
 struct alignas(16) SphTable { int n; int rule; int pad[2]; SphConst s[kMaxSph]; };         // rule: llq_config.knee_contacts
 
-// per-env shared-memory tables (floats)
-constexpr int kLinkTab = 12 * 8;      // link (3 k + i): c1 s1 cy sy | p(3) | -
-constexpr int kLegTab = 4 * 48;       // leg k: dynamics phase F(18) Hrow(9) rhs(3) Ic(10) facc(6); rows phase W(18) L(3) dinv(3) qd(3)
-constexpr int kConW = 20, kConTab = kMaxCon * kConW;   // contact: leg depth | Pc(3) n(3) t1(3) t2(3) | dist mu lam0 lam
-constexpr int kLimTab = kMaxLim * 4;  // limit row: leg joint dir pen
-constexpr int kRowW = 12, kRowTab = 32 * kRowW;        // row: y(6) e(3) leg - -   (aliased by the 16 x 20 float scratch of the dynamics phase)
-constexpr int kEnvTab = 56;           // p_base(6) - - | Cholesky factor of the base block (21) - - - | joint targets (12) | actions (12)
-constexpr int kATabWarp = 32 * 32;     // Delassus coefficients of one WARP (its two envs' rows packed into 32 lanes): atab[col * 32 + lane]
+// ---- per-env shared-memory tables (floats): one block of kEnvFloats per env, split into six tables by env_tabs
+// link record 3 k + i (link i of leg k): its rotation Rx(c1, s1) Ry(cy, sy) and origin p in base coordinates
+namespace linkrec { constexpr int c1 = 0, s1 = 1, cy = 2, sy = 3, p = 4, end = 7; }
+constexpr int kLinkW = 8, kLinkTab = 12 * kLinkW;
+// leg table of leg k, in two layouts.  Dynamics phase: column F_i of the coupling block (angular 3 | linear 3) at F + 6 i, row i of H_k
+// at H + 3 i, the joints' right-hand sides, and the leg's composite mass, first moment, inertia (xx xy xz yy yz zz) and bias wrench
+// (angular 3 | linear 3).  Rows phase, from the end of the forward dynamics on: column m of W = F L^-T at W + 6 m, L (L10 L20 L21),
+// D^-1, the predicted joint velocities, and the knee joint's c3, s3 for the fp64 clearance of the shank's spheres.
+namespace legdyn { constexpr int F = 0, H = 18, rhs = 27, m = 30, h = 31, Ic = 34, bias = 40, end = 46; }
+namespace legrow { constexpr int W = 0, L = 18, dinv = 21, qd = 24, c3 = 28, s3 = 29, end = 30; }
+constexpr int kLegW = 48, kLegTab = 4 * kLegW;
+static_assert(legdyn::end <= kLegW && legrow::end <= kLegW, "each phase of the leg table fits its 48 floats");
+// contact record: leg (-1: the base) and depth of the sphere's link (int bits), contact point, normal n and tangents t1 t2 (base
+// coordinates), clearance, friction, warm-start impulse, final normal impulse
+namespace conrec { constexpr int leg = 0, depth = 1, Pc = 2, n = 5, t1 = 8, t2 = 11, dist = 14, mu = 15, lam0 = 16, lam = 17, end = 18; }
+constexpr int kConW = 20, kConTab = kMaxCon * kConW;
+static_assert(conrec::t1 == conrec::n + 3 && conrec::t2 == conrec::n + 6, "row_image reads direction d at n + 3 d");
+static_assert(conrec::depth == conrec::leg + 1 && conrec::Pc == conrec::depth + 1 && conrec::n == conrec::Pc + 3 && conrec::dist == conrec::t2 + 3 &&
+              conrec::mu == conrec::dist + 1 && conrec::leg % 4 == 0 && conrec::end <= kConW && kConW % 4 == 0,
+              "the contact writer stores leg .. mu as four float4");
+// limit row: leg, joint (int bits), direction, penetration
+namespace limrec { constexpr int leg = 0, joint = 1, dir = 2, pen = 3; }
+constexpr int kLimW = 4, kLimTab = kMaxLim * kLimW;
+static_assert(limrec::joint == limrec::leg + 1 && limrec::dir == limrec::leg + 2 && limrec::pen == limrec::leg + 3 && limrec::leg == 0,
+              "the limit writer stores a row as one float4");
+// constraint row: its image y, e = D^-1 w and leg (int bits), for the other rows' Delassus entries
+namespace rowrec { constexpr int y = 0, e = 6, leg = 9; }
+constexpr int kRowW = 12, kRowTab = 32 * kRowW;
+static_assert(rowrec::y == 0 && rowrec::e == rowrec::y + 6 && rowrec::leg == rowrec::e + 3 && kRowW == 12,
+              "rows are moved as three float4: y0-3 | y4 y5 e0 e1 | e2 leg - -");
+// The row table's storage is also, in turn: the dynamics phase's scratch (one record of kScrW floats per lane), the solver's totals
+// (the impulse sums: base 6, then 3 per leg) and the hand-over to the step tail (TailState).
+constexpr int kScrW = 20;
+static_assert(16 * kScrW <= kRowTab, "the dynamics scratch lives in the row table");
+namespace sums { constexpr int base = 0, leg = 6, end = 18; }
+static_assert(sums::leg == sums::base + 6 && sums::end == sums::leg + 3 * 4 && sums::end <= kRowTab, "the impulse sums live in the row table");
+// env table: the base body's bias wrench (dynamics), which then becomes the predicted base velocity (rows) | packed Cholesky factor of
+// the base block | joint targets | actions
+namespace envslot { constexpr int bias = 0, vel = 0, chol = 8, target = 32, act = 44; }
+constexpr int kEnvTab = 56;
+static_assert(envslot::bias + 6 <= envslot::chol && envslot::chol + 21 <= envslot::target && envslot::target + kActDim <= envslot::act &&
+              envslot::act + kActDim <= kEnvTab, "env table slots");
 constexpr int kEnvFloats = 944;        // >= the sum of the tables, and = 16 (mod 32): envs an odd number of slots apart hit disjoint banks
 static_assert(kLinkTab + kLegTab + kConTab + kLimTab + kRowTab + kEnvTab <= kEnvFloats && kEnvFloats % 32 == 16, "per-env table layout");
+struct EnvTabs { float *link, *leg, *con, *lim, *row, *env; };
+LLQ_DI EnvTabs env_tabs(float* block) {          // block = s_env_dyn + e * kEnvFloats
+  EnvTabs t;
+  t.link = block; t.leg = t.link + kLinkTab; t.con = t.leg + kLegTab; t.lim = t.con + kConTab; t.row = t.lim + kLimTab; t.env = t.row + kRowTab;
+  return t;
+}
+// Delassus coefficients of one WARP (its two envs' rows packed into 32 lanes): column col of lane l at col * stride + l.  Contact c,
+// direction d -> column con + 3 c + d; limit row t -> column lim + t.
+namespace dcol { constexpr int con = 0, lim = 3 * kMaxCon, n = lim + kMaxLim, stride = 32; }
+constexpr int kATabWarp = dcol::n * dcol::stride;
+// staging-row borrows before the tail: the corridor's candidate boxes (6 floats each) and the SEPMC proxy points of each leg (foot |
+// knee wheel | hip | two body corners | handle, 3 floats each)
+constexpr int kProxyW = 18;
+static_assert(6 * kMaxCand <= kNewObs && 4 * kProxyW <= kNewObs, "the candidate boxes and the proxy points fit a staging row");
 
 LLQ_DI V3 rotxy(V3 v, float cy, float sy, float cx, float sx) { return rot<0>(rot<1>(v, cy, sy), cx, sx); }     // Rx Ry v
 LLQ_DI V3 rotxyT(V3 v, float cy, float sy, float cx, float sx) { return rotT<1>(rotT<0>(v, cx, sx), cy, sy); }  // (Rx Ry)^T v
@@ -166,7 +214,7 @@ struct RowsIn {
   int lane;             // 0..31
   int split;            // warp-uniform: 16 = every row on its own env's half-warp
   int Cmax, Lmax;       // warp-uniform maxima over the envs of this pass: contacts, limit rows
-  float* res;           // where the totals of the env behind this lane's HALF-warp go (18 floats at the head of its row table), or
+  float* res;           // where the totals of the env behind this lane's HALF-warp go (the impulse sums, at the head of its row table), or
                         // nullptr when that env is not solved in this pass
   float dt, slop, erp, jerp, max_imp;
   int iters;
@@ -176,12 +224,7 @@ struct RowRegs { float y[6], wj[3], b, rhs, invd, lam, hi, mu; int leg; };
 // row rr of the env behind in.tb: contact rr / 3 in direction rr % 3, or limit row rr - 3 nc; also leaves (y, e = D^-1 w, leg) in the
 // env's row table for the other rows' Delassus entries.  Returns true for a normal row (its impulse is the contact's warm start).
 LLQ_DI bool row_image(const RowsIn& in, RowRegs& r) {
-  const float* linktab = in.tb;
-  const float* legtab = in.tb + kLinkTab;
-  const float* contab = legtab + kLegTab;
-  const float* limtab = contab + kConTab;
-  float* rowtab = in.tb + kLinkTab + kLegTab + kConTab + kLimTab;
-  const float* envtab = rowtab + kRowTab;
+  const EnvTabs tab = env_tabs(in.tb);
   const int rr = in.rr;
   const bool is_con = rr < 3 * in.nc;
   const int d = rr % 3, cq = rr / 3;
@@ -196,42 +239,43 @@ LLQ_DI bool row_image(const RowsIn& in, RowRegs& r) {
     float j[3] = {0.f, 0.f, 0.f}, rel = 0.f, dist = 0.f, lam0 = 0.f, pen = 0.f, dirl = 0.f;
     int leg, jj = 0;
     if (is_con) {
-      const float* cr = contab + cq * kConW;
-      leg = __float_as_int(cr[0]);
-      const int depth = __float_as_int(cr[1]);
-      const V3 Pc = ld3(cr + 2), dir = ld3(cr + 5 + 3 * d);
-      dist = cr[14]; r.mu = cr[15]; lam0 = cr[16];
+      const float* cr = tab.con + cq * kConW;
+      leg = __float_as_int(cr[conrec::leg]);
+      const int depth = __float_as_int(cr[conrec::depth]);
+      const V3 Pc = ld3(cr + conrec::Pc), dir = ld3(cr + conrec::n + 3 * d);
+      dist = cr[conrec::dist]; r.mu = cr[conrec::mu]; lam0 = cr[conrec::lam0];
       Ga = cross(Pc, dir); Gl = dir;
-      rel = dot(Ga, ld3(envtab)) + dot(Gl, ld3(envtab + 3));     // predicted base velocity (base coordinates), parked by the env's lane 0
+      // predicted base velocity (base coordinates), parked by the env's lane 0
+      rel = dot(Ga, ld3(tab.env + envslot::vel)) + dot(Gl, ld3(tab.env + envslot::vel + 3));
       if (leg >= 0) {
-        const float* lk = linktab + leg * 24;
-        const float c1 = lk[0], s1 = lk[1];
-        const V3 p1 = ld3(lk + 4), p2 = ld3(lk + 12), p3 = ld3(lk + 20), n2 = V3{0.f, -c1, -s1};
+        const float* lk = tab.link + 3 * leg * kLinkW;     // links 0, 1, 2 of the leg
+        const float c1 = lk[linkrec::c1], s1 = lk[linkrec::s1];
+        const V3 p1 = ld3(lk + linkrec::p), p2 = ld3(lk + kLinkW + linkrec::p), p3 = ld3(lk + 2 * kLinkW + linkrec::p), n2 = V3{0.f, -c1, -s1};
         j[0] = Ga.x + dot(cross(p1, V3{1.f, 0.f, 0.f}), Gl);
         if (depth >= 2) j[1] = dot(n2, Ga) + dot(cross(p2, n2), Gl);
         if (depth >= 3) j[2] = dot(n2, Ga) + dot(cross(p3, n2), Gl);
       }
     } else {
-      const float* lr = limtab + (rr - 3 * in.nc) * 4;
-      leg = __float_as_int(lr[0]); jj = __float_as_int(lr[1]); dirl = lr[2]; pen = lr[3];
+      const float* lr = tab.lim + (rr - 3 * in.nc) * kLimW;
+      leg = __float_as_int(lr[limrec::leg]); jj = __float_as_int(lr[limrec::joint]); dirl = lr[limrec::dir]; pen = lr[limrec::pen];
       j[0] = jj == 0 ? dirl : 0.f; j[1] = jj == 1 ? dirl : 0.f; j[2] = jj == 2 ? dirl : 0.f;
     }
     r.leg = leg;
     float g[6] = {Ga.x, Ga.y, Ga.z, Gl.x, Gl.y, Gl.z};
     if (leg >= 0) {
-      const float* lt = legtab + leg * 48;
-      const float L10 = lt[18], L20 = lt[19], L21 = lt[20];
-      rel += j[0] * lt[24] + j[1] * lt[25] + j[2] * lt[26];
+      const float* lt = tab.leg + leg * kLegW;
+      const float L10 = lt[legrow::L], L20 = lt[legrow::L + 1], L21 = lt[legrow::L + 2];
+      rel += j[0] * lt[legrow::qd] + j[1] * lt[legrow::qd + 1] + j[2] * lt[legrow::qd + 2];
       r.wj[0] = j[0];
       r.wj[1] = fmaf(-L10, r.wj[0], j[1]);
       r.wj[2] = fmaf(-L20, r.wj[0], fmaf(-L21, r.wj[1], j[2]));
-      e[0] = r.wj[0] * lt[21]; e[1] = r.wj[1] * lt[22]; e[2] = r.wj[2] * lt[23];
+      e[0] = r.wj[0] * lt[legrow::dinv]; e[1] = r.wj[1] * lt[legrow::dinv + 1]; e[2] = r.wj[2] * lt[legrow::dinv + 2];
 #pragma unroll
       for (int m = 0; m < 3; m++)
 #pragma unroll
-        for (int t = 0; t < 6; t++) g[t] = fmaf(-e[m], lt[6 * m + t], g[t]);
+        for (int t = 0; t < 6; t++) g[t] = fmaf(-e[m], lt[legrow::W + 6 * m + t], g[t]);
     }
-    chol6_fwd_p(envtab + 8, g, r.y);
+    chol6_fwd_p(tab.env + envslot::chol, g, r.y);
     const float dg = dot6(r.y, r.y) + r.wj[0] * e[0] + r.wj[1] * e[1] + r.wj[2] * e[2];
     r.invd = 1.0f / dg;
     if (is_con) {
@@ -249,7 +293,7 @@ LLQ_DI bool row_image(const RowsIn& in, RowRegs& r) {
       r.rhs = (poserr - rel) * r.invd;
       r.hi = in.max_imp;
     }
-    float* rw = rowtab + rr * kRowW;
+    float* rw = tab.row + rr * kRowW + rowrec::y;
     st4(rw, r.y[0], r.y[1], r.y[2], r.y[3]);
     st4(rw + 4, r.y[4], r.y[5], e[0], e[1]);
     st4(rw + 8, e[2], __int_as_float(r.leg), 0.f, 0.f);
@@ -266,19 +310,19 @@ LLQ_DI float delassus_entry(const RowRegs& r, const float* rw) {
 // total impulse of an env: Yt += sum lam_r y_r and, per leg, sum lam_r w_r -- 18 values.  Rows that sit on the partner's half-warp are
 // handed across first (xor 16), then a butterfly over each half-warp.
 LLQ_DI void impulse_sums(const RowsIn& in, const RowRegs& r) {
-  float v18[18];
+  float v18[sums::end];
 #pragma unroll
-  for (int t = 0; t < 6; t++) v18[t] = r.lam * r.y[t];
+  for (int t = 0; t < 6; t++) v18[sums::base + t] = r.lam * r.y[t];
 #pragma unroll
   for (int kk = 0; kk < 4; kk++) {
     const float f = r.leg == kk ? r.lam : 0.f;
 #pragma unroll
-    for (int m = 0; m < 3; m++) v18[6 + 3 * kk + m] = f * r.wj[m];
+    for (int m = 0; m < 3; m++) v18[sums::leg + 3 * kk + m] = f * r.wj[m];
   }
   if (in.split != 16) {                                     // warp-uniform
     const bool foreign = (in.lane >= 16) != (in.lane >= in.split);      // the row belongs to the other half-warp's env
 #pragma unroll
-    for (int t = 0; t < 18; t++) {                          // (unrolled: a rolled loop would index v18 in local memory)
+    for (int t = 0; t < sums::end; t++) {                   // (unrolled: a rolled loop would index v18 in local memory)
       const float mine = foreign ? 0.f : v18[t], give = foreign ? v18[t] : 0.f;
       v18[t] = mine + __shfl_xor_sync(FULL, give, 16);
     }
@@ -286,12 +330,13 @@ LLQ_DI void impulse_sums(const RowsIn& in, const RowRegs& r) {
 #pragma unroll 1
   for (int o = 1; o < 16; o <<= 1) {
 #pragma unroll
-    for (int t = 0; t < 18; t++) v18[t] += __shfl_xor_sync(FULL, v18[t], o);
+    for (int t = 0; t < sums::end; t++) v18[t] += __shfl_xor_sync(FULL, v18[t], o);
   }
   if (in.res && (in.lane & 15) == 0) {                    // the lower half-warp holds env A's totals, the upper one env B's
-    st4(in.res, v18[0], v18[1], v18[2], v18[3]); st4(in.res + 4, v18[4], v18[5], v18[6], v18[7]);
-    st4(in.res + 8, v18[8], v18[9], v18[10], v18[11]); st4(in.res + 12, v18[12], v18[13], v18[14], v18[15]);
-    in.res[16] = v18[16]; in.res[17] = v18[17];
+#pragma unroll
+    for (int t = 0; t + 4 <= sums::end; t += 4) st4(in.res + t, v18[t], v18[t + 1], v18[t + 2], v18[t + 3]);
+#pragma unroll
+    for (int t = sums::end & ~3; t < sums::end; t++) in.res[t] = v18[t];
   }
 }
 
@@ -304,28 +349,28 @@ LLQ_DI void solve_rows(const RowsIn& in) {
   T16_IN(8);
   float* acol = in.acol;
   const int lane0 = in.lane0, nc = in.nc, nl = in.nl;
-  // Coefficient columns: contact c, direction d -> column 3 c + d (0..23); limit row t -> column 24 + t.  Columns the sweep visits
+  // Coefficient columns (dcol): contact c, direction d -> column con + 3 c + d; limit row t -> column lim + t.  Columns the sweep visits
   // for the partner's sake (its lists are longer) hold zeros, so that those steps change nothing; the loop bounds are rounded up to
   // even (the sweeps are unrolled by two; the caps are even).
   const int Ce = (in.Cmax + 1) & ~1, Le = (in.Lmax + 1) & ~1;
   {
-    const float* rowtab = in.tb + kLinkTab + kLegTab + kConTab + kLimTab;
+    const float* rowtab = env_tabs(in.tb).row;
     const int ncon = 3 * nc;
 #pragma unroll 1
     for (int col = 0; col < 3 * Ce; col++) {
       const float a = delassus_entry(r, rowtab + col * kRowW);
-      acol[col * 32] = col < ncon ? a : 0.f;        // (beyond the env's list the table holds old rows: finite, masked)
+      acol[(dcol::con + col) * dcol::stride] = col < ncon ? a : 0.f;        // (beyond the env's list the table holds old rows: finite, masked)
     }
     const float* rl = rowtab + ncon * kRowW;
 #pragma unroll 1
     for (int t = 0; t < Le; t++) {
       const float a = delassus_entry(r, rl + t * kRowW);
-      acol[(24 + t) * 32] = t < nl ? a : 0.f;
+      acol[(dcol::lim + t) * dcol::stride] = t < nl ? a : 0.f;
     }
   }
   // warm start of the normal rows
 #pragma unroll 1
-  for (int c = 0; c < in.Cmax; c++) r.b = fmaf(acol[96 * c], __shfl_sync(FULL, r.lam, lane0 + 3 * c), r.b);
+  for (int c = 0; c < in.Cmax; c++) r.b = fmaf(acol[(dcol::con + 3 * c) * dcol::stride], __shfl_sync(FULL, r.lam, lane0 + 3 * c), r.b);
   T16_IN(9);
   // projected Gauss-Seidel (btMultiBodyConstraintSolver::solveSingleIteration order).  One row update: candidate on every lane (only
   // the owner's counts), owner commits, broadcast, one LDS + FMA per lane.  Dependent chain per row: FFMA (candidate from
@@ -346,27 +391,27 @@ LLQ_DI void solve_rows(const RowsIn& in) {
   for (int it = 0; it < in.iters; it++) {
     {
       int src = lane0 + 3 * nc;
-      const float* ap = acol + 24 * 32;
+      const float* ap = acol + dcol::lim * dcol::stride;
 #pragma unroll 1
-      for (int t = 0; t < Le; t += 2, src += 2, ap += 64) {     // joint-limit rows in joint order
+      for (int t = 0; t < Le; t += 2, src += 2, ap += 2 * dcol::stride) {     // joint-limit rows in joint order
         LLQ16_ROW_UPDATE(src, ap[0], t < nl, LLQ16_CLAMP_LIMIT)
-        LLQ16_ROW_UPDATE(src + 1, ap[32], t + 1 < nl, LLQ16_CLAMP_LIMIT)
+        LLQ16_ROW_UPDATE(src + 1, ap[dcol::stride], t + 1 < nl, LLQ16_CLAMP_LIMIT)
       }
     }
     {
       int src = lane0;
-      const float* ap = acol;
+      const float* ap = acol + dcol::con * dcol::stride;
 #pragma unroll 1
-      for (int t = 0; t < Ce; t += 2, src += 6, ap += 192) {    // normal rows in contact order
+      for (int t = 0; t < Ce; t += 2, src += 6, ap += 6 * dcol::stride) {    // normal rows in contact order
         LLQ16_ROW_UPDATE(src, ap[0], t < nc, LLQ16_CLAMP_NORMAL)
-        LLQ16_ROW_UPDATE(src + 3, ap[96], t + 1 < nc, LLQ16_CLAMP_NORMAL)
+        LLQ16_ROW_UPDATE(src + 3, ap[3 * dcol::stride], t + 1 < nc, LLQ16_CLAMP_NORMAL)
       }
     }
     {
       int src = lane0;
-      const float* ap = acol;
+      const float* ap = acol + dcol::con * dcol::stride;
 #pragma unroll 1
-      for (int t = 0; t < in.Cmax; t++, src += 3, ap += 96) {   // friction pairs with the implicit cone (resolveConeFrictionConstraintRows)
+      for (int t = 0; t < in.Cmax; t++, src += 3, ap += 3 * dcol::stride) {   // friction pairs with the implicit cone (resolveConeFrictionConstraintRows)
         // One shuffle round trip on the dependent chain: the two tangent rows' candidates go to every lane together with their current
         // impulses and the cone's radius (those three do not depend on this step's b), and every lane forms both increments itself.
         const float sown = fmaf(-r.b, r.invd, rc);
@@ -381,7 +426,7 @@ LLQ_DI void solve_rows(const RowsIn& in) {
         const bool valid = t < nc;
         if (lane == src + 1 && valid) { r.lam = na; rc = na + r.rhs; }
         if (lane == src + 2 && valid) { r.lam = nb; rc = nb + r.rhs; }
-        r.b = fmaf(ap[32], na - la, fmaf(ap[64], nb - lb, r.b));
+        r.b = fmaf(ap[dcol::stride], na - la, fmaf(ap[2 * dcol::stride], nb - lb, r.b));
       }
     }
   }
@@ -390,7 +435,7 @@ LLQ_DI void solve_rows(const RowsIn& in) {
 #undef LLQ16_CLAMP_NORMAL
   T16_IN(10);
   // the normal impulses go back to the contact records (warm start of the next sub-step)
-  if (is_normal) in.tb[kLinkTab + kLegTab + (in.rr / 3) * kConW + 17] = r.lam;
+  if (is_normal) env_tabs(in.tb).con[(in.rr / 3) * kConW + conrec::lam] = r.lam;
   __syncwarp();                     // every lane is done with the row table: its head becomes the result area
   impulse_sums(in, r);
 }
@@ -402,9 +447,10 @@ LLQ_DI void solve_rows(const RowsIn& in) {
 // envs; here one instruction stream serves eight.
 struct TailState {            // per env, written by the env's lane 0 (base part) and its lanes (k, 0) (joint part)
   double px, py, pz, time, frame_frac;
-  int frame_id, ob_id, flags, push_count, push_draws;      // flags: bad | ob_hit << 1 | touch_own << 2 | tag << 3
+  int frame_id, ob_id, flags, push_count, push_draws;      // flags: tflag bits
   float pf[3], qp[4], vw[3], ww[3], q[12], qd[12];
 };
+namespace tflag { constexpr int bad = 1, ob_hit = 2, touch_own = 4, tag = 8; }
 static_assert(sizeof(TailState) <= sizeof(float) * kRowTab, "the hand-over record lives in the row table");
 template <int ENV>
 LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& P, const ModelConst& M, float* s_new, const float* s_hist,
@@ -413,8 +459,8 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
   const int N = P.n_envs;
   double px = T.px, py = T.py, pz = T.pz, time = T.time, frame_frac = T.frame_frac;
   int frame_id = T.frame_id, ob_id = T.ob_id, push_count = T.push_count, push_draws = T.push_draws;
-  bool bad = (T.flags & 1) != 0, ob_hit = (T.flags & 2) != 0;
-  const bool touch_own = (T.flags & 4) != 0, tag = (T.flags & 8) != 0;
+  bool bad = (T.flags & tflag::bad) != 0, ob_hit = (T.flags & tflag::ob_hit) != 0;
+  const bool touch_own = (T.flags & tflag::touch_own) != 0, tag = (T.flags & tflag::tag) != 0;
   const float pf[3] = {T.pf[0], T.pf[1], T.pf[2]};
   const Q4 qp = Q4{T.qp[0], T.qp[1], T.qp[2], T.qp[3]};
   const V3 vw = V3{T.vw[0], T.vw[1], T.vw[2]}, ww = V3{T.ww[0], T.ww[1], T.ww[2]};
@@ -480,13 +526,14 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
     if (wr) {
       store_state(E, N, env, k, q, qd, fd, px, py, pz, qb, vw, ww);
 #pragma unroll
-      for (int t = 0; t < 3; t++) { E.kin[(13 + 3 * k + t) * N + env] = oc.kq[t]; E.kin[(25 + 3 * k + t) * N + env] = oc.kqd[t]; }
+      for (int t = 0; t < 3; t++) { E.kin[(state::q + 3 * k + t) * N + env] = oc.kq[t]; E.kin[(state::qd + 3 * k + t) * N + env] = oc.kqd[t]; }
       if (k == 0) {
         if (P.has_ob) E.ob_id[env] = ob_id;
-        E.kin[env] = (float)oc.kb.px; E.kin[N + env] = (float)oc.kb.py; E.kin[2 * N + env] = (float)oc.kb.pz;
-        E.kin[3 * N + env] = oc.kb.q.x; E.kin[4 * N + env] = oc.kb.q.y; E.kin[5 * N + env] = oc.kb.q.z; E.kin[6 * N + env] = oc.kb.q.w;
-        E.kin[7 * N + env] = oc.kb.lin.x; E.kin[8 * N + env] = oc.kb.lin.y; E.kin[9 * N + env] = oc.kb.lin.z;
-        E.kin[10 * N + env] = oc.kb.ang.x; E.kin[11 * N + env] = oc.kb.ang.y; E.kin[12 * N + env] = oc.kb.ang.z;
+        E.kin[state::pos * N + env] = (float)oc.kb.px; E.kin[(state::pos + 1) * N + env] = (float)oc.kb.py; E.kin[(state::pos + 2) * N + env] = (float)oc.kb.pz;
+        E.kin[state::quat * N + env] = oc.kb.q.x; E.kin[(state::quat + 1) * N + env] = oc.kb.q.y;
+        E.kin[(state::quat + 2) * N + env] = oc.kb.q.z; E.kin[(state::quat + 3) * N + env] = oc.kb.q.w;
+        E.kin[state::lin * N + env] = oc.kb.lin.x; E.kin[(state::lin + 1) * N + env] = oc.kb.lin.y; E.kin[(state::lin + 2) * N + env] = oc.kb.lin.z;
+        E.kin[state::ang * N + env] = oc.kb.ang.x; E.kin[(state::ang + 1) * N + env] = oc.kb.ang.y; E.kin[(state::ang + 2) * N + env] = oc.kb.ang.z;
         if (done) {
           E.done_reward[env] = E.reward_sum[env] + rew;
           atomicMax(&winner[clip], env);       // highest finished env index owns the clip's slot this step (PLE:236)
@@ -621,7 +668,7 @@ LLQ_DI void step_tail(const EnvArrays& E, const MocapDev& mc, const StepParams& 
     float* row = obs2 + (size_t)env * obs2_ld + ObsW<ENV>::value - (record == 2 ? (long long)N * obs2_ld : 0ll);
 #pragma unroll
     for (int t = 0; t < 3; t++) row[3 * k + t] = act_src[3 * k + t];
-    if (k == 0) { row[12] = rew_out; row[13] = done ? 1.f : 0.f; }
+    if (k == 0) { row[kRecReward] = rew_out; row[kRecDone] = done ? 1.f : 0.f; }
   }
   {
     const unsigned dm = __ballot_sync(FULL, valid && k == 0 && done);       // episodes finished: one atomic per warp
@@ -666,15 +713,16 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
   const bool valid = env_raw < N;
   const LegConst& L = M.leg[k];
   const V3 r0 = ld3(L.j[0].r), r1 = ld3(L.j[1].r), r2 = ld3(L.j[2].r);
+  // this env's tables, the env_tabs split spelled out: taking the same pointers from an EnvTabs changes ptxas's schedule of this kernel
   float* const linktab = s_env_dyn + el * kEnvFloats;
   float* const legtab = linktab + kLinkTab;
   float* const contab = legtab + kLegTab;
   float* const limtab = contab + kConTab;
   float* const rowtab = limtab + kLimTab;
-  float* const scr = rowtab;                         // dynamics-phase scratch (16 lanes x 20 floats) aliases the row table
+  float* const scr = rowtab;                         // dynamics-phase scratch (16 lanes x kScrW floats) aliases the row table
   float* const envtab = rowtab + kRowTab;
-  float* const s_atab = s_env_dyn + EPB * kEnvFloats;   // [BLOCK / 32][32 cols][32 lanes] Delassus coefficients, one table per warp
-  for (int col = 0; col < 32; col++) s_atab[(tid >> 5) * kATabWarp + col * 32 + (tid & 31)] = 0.f;      // finite from the start (masked steps multiply them by 0)
+  float* const s_atab = s_env_dyn + EPB * kEnvFloats;   // [BLOCK / 32][dcol::n][32 lanes] Delassus coefficients, one table per warp
+  for (int col = 0; col < dcol::n; col++) s_atab[(tid >> 5) * kATabWarp + col * dcol::stride + (tid & 31)] = 0.f;      // finite from the start (masked steps multiply them by 0)
   // joints with a lower dof index than this lane's (k, i): rank of a violated limit in Bullet's row order
   unsigned lowmask = 0;
 #pragma unroll
@@ -682,20 +730,20 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
 
   // ---- load state (base entries replicated on the 16 lanes, joint entries on the 4 lanes of the leg)
   double px = E.pos[env], py = E.pos[N + env], pz = E.pos[2 * N + env];
-  const float* st = E.st;
-  Q4 qb = Q4{st[env], st[N + env], st[2 * N + env], st[3 * N + env]};
-  V3 vw = V3{st[4 * N + env], st[5 * N + env], st[6 * N + env]};
-  V3 ww = V3{st[7 * N + env], st[8 * N + env], st[9 * N + env]};
+  const float* sr = E.st;
+  Q4 qb = Q4{sr[st::quat * N + env], sr[(st::quat + 1) * N + env], sr[(st::quat + 2) * N + env], sr[(st::quat + 3) * N + env]};
+  V3 vw = V3{sr[st::lin * N + env], sr[(st::lin + 1) * N + env], sr[(st::lin + 2) * N + env]};
+  V3 ww = V3{sr[st::ang * N + env], sr[(st::ang + 1) * N + env], sr[(st::ang + 2) * N + env]};
   float q[3], qd[3];
 #pragma unroll
   for (int t = 0; t < 3; t++) {
-    q[t] = st[(10 + 3 * k + t) * N + env];
-    qd[t] = st[(22 + 3 * k + t) * N + env];
+    q[t] = sr[(st::q + 3 * k + t) * N + env];
+    qd[t] = sr[(st::qd + 3 * k + t) * N + env];
   }
   if (i < 3) {                                               // joint (k, i): action and clipped target stay in shared memory
     const float a = actions[(size_t)env * kActDim + 3 * k + i];
-    envtab[44 + 3 * k + i] = a;
-    envtab[32 + 3 * k + i] = clampf((i == 0 ? q[0] : (i == 1 ? q[1] : q[2])) + a, -3.0f, 3.0f);           // PLE:200, LR:126-127
+    envtab[envslot::act + 3 * k + i] = a;
+    envtab[envslot::target + 3 * k + i] = clampf((i == 0 ? q[0] : (i == 1 ? q[1] : q[2])) + a, -3.0f, 3.0f);           // PLE:200, LR:126-127
   }
   const int nsph = ST.n, rule = ST.rule;
   float warm[2];                                             // remembered normal impulses of spheres l16 and l16 + 16
@@ -726,7 +774,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
   int n_cand = 0;
   float* s_cand = nullptr;
   if (ENV == kEpmcCorridor) {
-    s_cand = &s_new[el][0];                            // the staging row is free until the tail: 8 x 6 floats
+    s_cand = &s_new[el][0];                            // the staging row is free until the tail: kMaxCand x 6 floats
     const float* bxs = E.boxes + (size_t)env * (6 * kMaxBoxes);
     // reach of the robot's spheres from the base reference point: hip offset 0.195 + leg 0.48 in x, 0.15 + 0.05 in y, plus the
     // travel during the step (<= 0.06 m at 3 m/s) -> 0.8 m per axis (0.6 missed hind feet stretched backwards over a hurdle)
@@ -745,7 +793,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     __syncwarp();
   }
   // base orientation: pybullet speaks in the base inertial frame; dynamics run in URDF body axes B' = inertial * qI^-1
-  const Q4 qI = Q4{M.base.qI[0], M.base.qI[1], M.base.qI[2], M.base.qI[3]};
+  const Q4 qI = base_qI(M);
   Q4 qp = qmul(qnormalize(qb), qconj(qI));
   unsigned n_contact_rows = 0, n_limit_rows = 0, n_overflow = 0;
   bool bad = false;
@@ -838,14 +886,14 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     }
     // ---------------- composite inertia / accumulated bias wrench along the leg (suffix sums through the scratch rows)
     {
-      float* my = scr + l16 * 20;
+      float* my = scr + l16 * kScrW;
       st4(my, f.a.x, f.a.y, f.a.z, f.l.x); st4(my + 4, f.l.y, f.l.z, mc_, hc.x);
       st4(my + 8, hc.y, hc.z, Ic.xx, Ic.xy); st4(my + 12, Ic.xz, Ic.yy, Ic.yz, Ic.zz);
       __syncwarp();
       if (i < 2) {
 #pragma unroll 1
         for (int up = i + 1; up < 3; up++) {
-          const float* o = scr + (k + 4 * up) * 20;
+          const float* o = scr + (k + 4 * up) * kScrW;
           const float4 a = ld4(o), b4 = ld4(o + 4), c4 = ld4(o + 8), d4 = ld4(o + 12);
           f.a = f.a + V3{a.x, a.y, a.z}; f.l = f.l + V3{a.w, b4.x, b4.y};
           mc_ += b4.z; hc = hc + V3{b4.w, c4.x, c4.y};
@@ -860,22 +908,26 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
       const float Cb = dot(ax, f.a) + dot(al, f.l);
       const float h0 = Fa.x + dot(l1, Fl), h1 = dot(n2, Fa) + dot(l2, Fl), h2 = dot(n2, Fa) + dot(l3, Fl);
       const float qi = i == 0 ? q[0] : (i == 1 ? q[1] : q[2]), qdi = i == 0 ? qd[0] : (i == 1 ? qd[1] : qd[2]);
-      const float tg = envtab[32 + 3 * k + ic];
+      const float tg = envtab[envslot::target + 3 * k + ic];
       const float tau = clampf(fmaf(P.kp, tg - qi, P.kd * (0.f - qdi)), -P.max_tau, P.max_tau) - L.j[ic].jdamp * qdi;
-      float* lt = legtab + k * 48;
+      float* lt = legtab + k * kLegW;
       if (i < 3) {
-        lt[6 * i] = Fa.x; lt[6 * i + 1] = Fa.y; lt[6 * i + 2] = Fa.z; lt[6 * i + 3] = Fl.x; lt[6 * i + 4] = Fl.y; lt[6 * i + 5] = Fl.z;
-        lt[18 + 3 * i] = h0; lt[19 + 3 * i] = h1; lt[20 + 3 * i] = h2;
-        lt[27 + i] = tau - Cb;
-        float* lk = linktab + (3 * k + i) * 8;
-        st4(lk, c1, s1, cy, sy); st4(lk + 4, po.x, po.y, po.z, 0.f);
+        float* Fi = lt + legdyn::F + 6 * i;
+        Fi[0] = Fa.x; Fi[1] = Fa.y; Fi[2] = Fa.z; Fi[3] = Fl.x; Fi[4] = Fl.y; Fi[5] = Fl.z;
+        lt[legdyn::H + 3 * i] = h0; lt[legdyn::H + 3 * i + 1] = h1; lt[legdyn::H + 3 * i + 2] = h2;
+        lt[legdyn::rhs + i] = tau - Cb;
+        float* lk = linktab + (3 * k + i) * kLinkW;
+        st4(lk + linkrec::c1, c1, s1, cy, sy); st4(lk + linkrec::p, po.x, po.y, po.z, 0.f);
         if (i == 0) {
-          lt[30] = mc_; lt[31] = hc.x; lt[32] = hc.y; lt[33] = hc.z;
-          lt[34] = Ic.xx; lt[35] = Ic.xy; lt[36] = Ic.xz; lt[37] = Ic.yy; lt[38] = Ic.yz; lt[39] = Ic.zz;
-          lt[40] = f.a.x; lt[41] = f.a.y; lt[42] = f.a.z; lt[43] = f.l.x; lt[44] = f.l.y; lt[45] = f.l.z;
+          lt[legdyn::m] = mc_; lt[legdyn::h] = hc.x; lt[legdyn::h + 1] = hc.y; lt[legdyn::h + 2] = hc.z;
+          float* Il = lt + legdyn::Ic;
+          Il[0] = Ic.xx; Il[1] = Ic.xy; Il[2] = Ic.xz; Il[3] = Ic.yy; Il[4] = Ic.yz; Il[5] = Ic.zz;
+          float* bw = lt + legdyn::bias;
+          bw[0] = f.a.x; bw[1] = f.a.y; bw[2] = f.a.z; bw[3] = f.l.x; bw[4] = f.l.y; bw[5] = f.l.z;
         }
       } else if (k == 0) {
-        envtab[0] = f.a.x; envtab[1] = f.a.y; envtab[2] = f.a.z; envtab[3] = f.l.x; envtab[4] = f.l.y; envtab[5] = f.l.z;
+        float* bw = envtab + envslot::bias;
+        bw[0] = f.a.x; bw[1] = f.a.y; bw[2] = f.a.z; bw[3] = f.l.x; bw[4] = f.l.y; bw[5] = f.l.z;
       }
     }
     __syncwarp();
@@ -883,12 +935,13 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     float W[3][6], L10, L20, L21, di[3], u[3];
     float m6[21], z0[6];
     {
-      const float* lt = legtab + k * 48;
+      const float* lt = legtab + k * kLegW;
 #pragma unroll
       for (int m = 0; m < 3; m++)
 #pragma unroll
-        for (int t = 0; t < 6; t++) W[m][t] = lt[6 * m + t];
-      const float H00 = lt[18], H10 = lt[21], H11 = lt[22], H20 = lt[24], H21 = lt[25], H22 = lt[26];
+        for (int t = 0; t < 6; t++) W[m][t] = lt[legdyn::F + 6 * m + t];
+      const float* H = lt + legdyn::H;                     // row i at 3 i
+      const float H00 = H[0], H10 = H[3], H11 = H[4], H20 = H[6], H21 = H[7], H22 = H[8];
       di[0] = 1.0f / H00;
       L10 = H10 * di[0]; L20 = H20 * di[0];
       const float d1 = fmaf(-L10, H10, H11);
@@ -902,13 +955,15 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
         W[1][t] = fmaf(-L10, W[0][t], W[1][t]);
         W[2][t] = fmaf(-L20, W[0][t], fmaf(-L21, W[1][t], W[2][t]));
       }
-      u[0] = lt[27]; u[1] = fmaf(-L10, u[0], lt[28]); u[2] = fmaf(-L20, u[0], fmaf(-L21, u[1], lt[29]));
-      const float cm = lt[30];
-      const V3 ch_ = ld3(lt + 31);
+      const float* rhs = lt + legdyn::rhs;
+      u[0] = rhs[0]; u[1] = fmaf(-L10, u[0], rhs[1]); u[2] = fmaf(-L20, u[0], fmaf(-L21, u[1], rhs[2]));
+      const float cm = lt[legdyn::m];
+      const V3 ch_ = ld3(lt + legdyn::h);
       const M3 hx = skew(ch_);
+      const float* Il = lt + legdyn::Ic;                   // xx xy xz yy yz zz
       // packed lower triangle of [[A, B], [B^T, C]] : rows 0-2 = A, rows 3-5 = [B^T, C]
-      m6[tri(0, 0)] = lt[34]; m6[tri(1, 0)] = lt[35]; m6[tri(1, 1)] = lt[37];
-      m6[tri(2, 0)] = lt[36]; m6[tri(2, 1)] = lt[38]; m6[tri(2, 2)] = lt[39];
+      m6[tri(0, 0)] = Il[0]; m6[tri(1, 0)] = Il[1]; m6[tri(1, 1)] = Il[3];
+      m6[tri(2, 0)] = Il[2]; m6[tri(2, 1)] = Il[4]; m6[tri(2, 2)] = Il[5];
       m6[tri(3, 0)] = hx.a00; m6[tri(3, 1)] = hx.a10; m6[tri(3, 2)] = hx.a20;
       m6[tri(4, 0)] = hx.a01; m6[tri(4, 1)] = hx.a11; m6[tri(4, 2)] = hx.a21;
       m6[tri(5, 0)] = hx.a02; m6[tri(5, 1)] = hx.a12; m6[tri(5, 2)] = hx.a22;
@@ -923,7 +978,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
           for (int c = 0; c <= r; c++) m6[tri(r, c)] = fmaf(-wd, W[m][c], m6[tri(r, c)]);
         }
 #pragma unroll
-        for (int t = 0; t < 6; t++) z0[t] = (m == 0 ? lt[40 + t] : z0[t]) + ud * W[m][t];
+        for (int t = 0; t < 6; t++) z0[t] = (m == 0 ? lt[legdyn::bias + t] : z0[t]) + ud * W[m][t];
       }
       // the four legs (xor 1, 2 stay inside the group of lanes with the same link index)
 #pragma unroll
@@ -939,7 +994,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
       m6[tri(5, 0)] += bx.a02; m6[tri(5, 1)] += bx.a12; m6[tri(5, 2)] += bx.a22;
       m6[tri(3, 3)] += bm; m6[tri(4, 4)] += bm; m6[tri(5, 5)] += bm;
 #pragma unroll
-      for (int t = 0; t < 6; t++) z0[t] += envtab[t];
+      for (int t = 0; t < 6; t++) z0[t] += envtab[envslot::bias + t];
     }
     float a0[6];
     {
@@ -950,7 +1005,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
       chol6_solve(ch, bneg, a0);                // acceleration relative to free fall (gravity as a fictitious base acceleration)
       if (l16 == 0) {                           // the factor is needed again by the row images and the final back substitution
 #pragma unroll
-        for (int t = 0; t < 21; t++) envtab[8 + t] = ch.l[t];
+        for (int t = 0; t < 21; t++) envtab[envslot::chol + t] = ch.l[t];
       }
     }
     // ---------------- joint accelerations of this lane's leg, velocity prediction v* = clamp(v + a dt)
@@ -972,17 +1027,19 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     wbs = tmul(R, ww); vbs = tmul(R, vw);
     __syncwarp();                                     // every lane has read F / H: the leg table becomes the rows' table
     if (l16 == 0) {                                   // predicted base velocity for the rows' right-hand sides (any lane of the warp may build them)
-      envtab[0] = wbs.x; envtab[1] = wbs.y; envtab[2] = wbs.z; envtab[3] = vbs.x; envtab[4] = vbs.y; envtab[5] = vbs.z;
+      float* v = envtab + envslot::vel;
+      v[0] = wbs.x; v[1] = wbs.y; v[2] = wbs.z; v[3] = vbs.x; v[4] = vbs.y; v[5] = vbs.z;
     }
     if (i == 0) {
-      float* lt = legtab + k * 48;
+      float* lt = legtab + k * kLegW;
 #pragma unroll
       for (int m = 0; m < 3; m++)
 #pragma unroll
-        for (int t = 0; t < 6; t++) lt[6 * m + t] = W[m][t];
-      lt[18] = L10; lt[19] = L20; lt[20] = L21; lt[21] = di[0]; lt[22] = di[1]; lt[23] = di[2];
-      lt[24] = qd[0]; lt[25] = qd[1]; lt[26] = qd[2];
-      lt[28] = c3; lt[29] = s3;                       // for the fp64 clearance of the shank's spheres
+        for (int t = 0; t < 6; t++) lt[legrow::W + 6 * m + t] = W[m][t];
+      lt[legrow::L] = L10; lt[legrow::L + 1] = L20; lt[legrow::L + 2] = L21;
+      lt[legrow::dinv] = di[0]; lt[legrow::dinv + 1] = di[1]; lt[legrow::dinv + 2] = di[2];
+      lt[legrow::qd] = qd[0]; lt[legrow::qd + 1] = qd[1]; lt[legrow::qd + 2] = qd[2];
+      lt[legrow::c3] = c3; lt[legrow::s3] = s3;       // for the fp64 clearance of the shank's spheres
     }
     }   // ================ end of the forward dynamics
     T16_MARK(1);
@@ -992,9 +1049,10 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     if (ENV == kPmc && P.has_ob && sub == P.substeps - 1) {
       const int o0 = mc.ob_off[clip], n_ob = mc.ob_off[clip + 1] - o0;
       if (n_ob > 0) {
-        const float* lk = linktab + 24 * k;
-        const float c1 = lk[0], s1 = lk[1], c2 = lk[10], s2 = lk[11], c23 = lk[18], s23 = lk[19];
-        const V3 p1 = ld3(lk + 4), p2 = ld3(lk + 12), p3 = ld3(lk + 20);
+        const float* lk = linktab + 3 * k * kLinkW;     // links 0, 1, 2 of the leg
+        const float c1 = lk[linkrec::c1], s1 = lk[linkrec::s1], c2 = lk[kLinkW + linkrec::cy], s2 = lk[kLinkW + linkrec::sy];
+        const float c23 = lk[2 * kLinkW + linkrec::cy], s23 = lk[2 * kLinkW + linkrec::sy];
+        const V3 p1 = ld3(lk + linkrec::p), p2 = ld3(lk + kLinkW + linkrec::p), p3 = ld3(lk + 2 * kLinkW + linkrec::p);
         const V3 fb = p3 + rot<0>(rot<1>(ld3(L.foot), c23, s23), c1, s1);     // foot centre of this lane's leg
         const double* ob = mc.ob_table + (size_t)(o0 + ob_id) * 4;
         float sy_, cy_;
@@ -1014,15 +1072,16 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
       float* srow = &s_new[el][0];
       const float* prow = &s_new[el ^ 1][0];
       const V3 pw = V3{(float)px, (float)py, (float)pz};
-      const float* lk = linktab + 24 * k;
-      const float c1 = lk[0], s1 = lk[1], c2 = lk[10], s2 = lk[11], c23 = lk[18], s23 = lk[19];
-      const V3 p1 = ld3(lk + 4), p2 = ld3(lk + 12), p3 = ld3(lk + 20);
+      const float* lk = linktab + 3 * k * kLinkW;       // links 0, 1, 2 of the leg
+      const float c1 = lk[linkrec::c1], s1 = lk[linkrec::s1], c2 = lk[kLinkW + linkrec::cy], s2 = lk[kLinkW + linkrec::sy];
+      const float c23 = lk[2 * kLinkW + linkrec::cy], s23 = lk[2 * kLinkW + linkrec::sy];
+      const V3 p1 = ld3(lk + linkrec::p), p2 = ld3(lk + kLinkW + linkrec::p), p3 = ld3(lk + 2 * kLinkW + linkrec::p);
       const V3 fb = p3 + rot<0>(rot<1>(ld3(L.foot), c23, s23), c1, s1);       // foot centre of this lane's leg
       const V3 wh = pw + mul(R, p2 + rot<0>(rot<1>(ld3(M.wheel_off[k]), c2, s2), c1, s1));
       const V3 hp_ = pw + mul(R, p1), ft = pw + mul(R, fb);
       const V3 c0 = pw + mul(R, ld3(M.corner[2 * k])), c1_ = pw + mul(R, ld3(M.corner[2 * k + 1]));
       if (i == 0) {
-        float* o = srow + 18 * k;
+        float* o = srow + kProxyW * k;
         o[0] = ft.x; o[1] = ft.y; o[2] = ft.z; o[3] = wh.x; o[4] = wh.y; o[5] = wh.z; o[6] = hp_.x; o[7] = hp_.y; o[8] = hp_.z;
         o[9] = c0.x; o[10] = c0.y; o[11] = c0.z; o[12] = c1_.x; o[13] = c1_.y; o[14] = c1_.z;
         if (k < 2) { const V3 hd = pw + mul(R, V3{M.handle[k][0], M.handle[k][1], M.handle[k][2]}); o[15] = hd.x; o[16] = hd.y; o[17] = hd.z; }
@@ -1034,7 +1093,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
       bool tg = false;
 #pragma unroll 1
       for (int j = 0; j < 4; j++) {
-        const float* pj = prow + 18 * j;
+        const float* pj = prow + kProxyW * j;
         const float rj[6] = {M.leg[j].foot_r, M.wheel_r[j], M.hip_r[j], 0.f, 0.f, M.handle[j & 1][3]};
 #pragma unroll
         for (int t = 0; t < 6; t++) {
@@ -1069,8 +1128,8 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
         float lc1 = 1.f, ls1 = 0.f, lcy = 1.f, lsy = 0.f;
         V3 lp = V3{0.f, 0.f, 0.f};
         if (sdep > 0) {
-          const float* lk = linktab + (3 * sleg + sdep - 1) * 8;
-          const float4 a = ld4(lk), b4 = ld4(lk + 4);
+          const float* lk = linktab + (3 * sleg + sdep - 1) * kLinkW;
+          const float4 a = ld4(lk + linkrec::c1), b4 = ld4(lk + linkrec::p);
           lc1 = a.x; ls1 = a.y; lcy = a.z; lsy = a.w; lp = V3{b4.x, b4.y, b4.z};
         }
         const V3 cl = ld3(sp.c);
@@ -1103,12 +1162,13 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
             if (sdep > 0) {
               const LegConst& SL = M.leg[sleg];
               if (sdep == 3) {
-                const double dc3 = (double)legtab[sleg * 48 + 28], ds3 = (double)legtab[sleg * 48 + 29];
+                const double dc3 = (double)legtab[sleg * kLegW + legrow::c3], ds3 = (double)legtab[sleg * kLegW + legrow::s3];
                 t = dc3 * x + ds3 * z; z = -ds3 * x + dc3 * z; x = t;            // Ry(theta3)
                 x += (double)SL.j[2].r[0]; y += (double)SL.j[2].r[1]; z += (double)SL.j[2].r[2];
               }
               if (sdep >= 2) {
-                const double dc2 = (double)linktab[(3 * sleg + 1) * 8 + 2], ds2 = (double)linktab[(3 * sleg + 1) * 8 + 3];
+                const float* l1 = linktab + (3 * sleg + 1) * kLinkW;
+                const double dc2 = (double)l1[linkrec::cy], ds2 = (double)l1[linkrec::sy];
                 t = dc2 * x + ds2 * z; z = -ds2 * x + dc2 * z; x = t;            // Ry(theta2)
                 x += (double)SL.j[1].r[0]; y += (double)SL.j[1].r[1]; z += (double)SL.j[1].r[2];
               }
@@ -1192,12 +1252,12 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
             dn = tmul(R, n); d1_ = tmul(R, t1); d2_ = tmul(R, t2);
           }
           const V3 Pc = cb - sp.r * dn;                   // contact point on the sphere surface
-          float* cr = contab + idx * kConW;
+          float* cr = contab + idx * kConW + conrec::leg;
           st4(cr, __int_as_float(sdep > 0 ? sleg : -1), __int_as_float(sdep), Pc.x, Pc.y);
           st4(cr + 4, Pc.z, dn.x, dn.y, dn.z);
           st4(cr + 8, d1_.x, d1_.y, d1_.z, d2_.x);
           st4(cr + 12, d2_.y, d2_.z, dist, sp.foot ? mu_foot : sp.mu_link);
-          cr[16] = P.warm * warm[rd]; cr[17] = 0.f;
+          cr[conrec::lam0] = P.warm * warm[rd]; cr[conrec::lam] = 0.f;
           mycon[rd] = idx;
         } else {
           warm[rd] = 0.f;                                 // manifold point removed: no warm start
@@ -1219,7 +1279,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
       nl = __popc(bal);
       const int rk = __popc(bal & lowmask);
       if (dir != 0.f) {
-        if (rk < kMaxLim) st4(limtab + rk * 4, __int_as_float(k), __int_as_float(i), dir, pen);
+        if (rk < kMaxLim) st4(limtab + rk * kLimW + limrec::leg, __int_as_float(k), __int_as_float(i), dir, pen);
         else n_overflow += 1;
       }
       if (nl > kMaxLim) nl = kMaxLim;
@@ -1274,7 +1334,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
           in.Cmax = two_pass ? (pass == 0 ? cA : cB) : max(cA, cB);
           in.Lmax = two_pass ? (pass == 0 ? lA : lB) : max(lA, lB);
           const bool upper = lane >= 16;
-          in.res = (two_pass && upper != (pass == 1)) ? nullptr : (upper ? tbB : tbA) + (kLinkTab + kLegTab + kConTab + kLimTab);
+          in.res = (two_pass && upper != (pass == 1)) ? nullptr : (upper ? tbB : tbA) + (rowtab - linktab);
           solve_rows(in);
           __syncwarp();
         }
@@ -1285,20 +1345,23 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     if (nc | nl) {
       if (l16 == 0) { n_contact_rows += 3u * (unsigned)nc; n_limit_rows += (unsigned)nl; }
 #pragma unroll
-      for (int rd = 0; rd < 2; rd++) if (mycon[rd] >= 0) warm[rd] = contab[mycon[rd] * kConW + 17];
+      for (int rd = 0; rd < 2; rd++) if (mycon[rd] >= 0) warm[rd] = contab[mycon[rd] * kConW + conrec::lam];
       // ---- total impulse -> velocity change: one back substitution for the base, one 3x3 solve per leg
-      const float4 y0 = ld4(rowtab), y1 = ld4(rowtab + 4);
+      const float* yt = rowtab + sums::base;
+      const float4 y0 = ld4(yt), y1 = ld4(yt + 4);
       const float Yt[6] = {y0.x, y0.y, y0.z, y0.w, y1.x, y1.y};
-      const float om[3] = {rowtab[6 + 3 * k], rowtab[7 + 3 * k], rowtab[8 + 3 * k]};
-      chol6_bwd_p(envtab + 8, Yt, dvb);
-      const float* lt = legtab + k * 48;            // W, L, D^-1 of this lane's leg come back from the leg table (not kept live across the solve)
+      const float om[3] = {rowtab[sums::leg + 3 * k], rowtab[sums::leg + 1 + 3 * k], rowtab[sums::leg + 2 + 3 * k]};
+      chol6_bwd_p(envtab + envslot::chol, Yt, dvb);
+      const float* lt = legtab + k * kLegW;        // W, L, D^-1 of this lane's leg come back from the leg table (not kept live across the solve)
       float t3[3];
 #pragma unroll
       for (int m = 0; m < 3; m++) {
-        const float wm[6] = {lt[6 * m], lt[6 * m + 1], lt[6 * m + 2], lt[6 * m + 3], lt[6 * m + 4], lt[6 * m + 5]};
-        t3[m] = (om[m] - dot6(wm, dvb)) * lt[21 + m];
+        const float wm[6] = {lt[legrow::W + 6 * m], lt[legrow::W + 6 * m + 1], lt[legrow::W + 6 * m + 2], lt[legrow::W + 6 * m + 3],
+                             lt[legrow::W + 6 * m + 4], lt[legrow::W + 6 * m + 5]};
+        t3[m] = (om[m] - dot6(wm, dvb)) * lt[legrow::dinv + m];
       }
-      dvl[2] = t3[2]; dvl[1] = fmaf(-lt[20], dvl[2], t3[1]); dvl[0] = fmaf(-lt[18], dvl[1], fmaf(-lt[19], dvl[2], t3[0]));
+      // L = (L10, L20, L21)
+      dvl[2] = t3[2]; dvl[1] = fmaf(-lt[legrow::L + 2], dvl[2], t3[1]); dvl[0] = fmaf(-lt[legrow::L], dvl[1], fmaf(-lt[legrow::L + 1], dvl[2], t3[0]));
     }
     __syncwarp();              // the row table is the next sub-step's scratch
     T16_MARK(3);
@@ -1355,7 +1418,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
       T->vw[0] = vw.x; T->vw[1] = vw.y; T->vw[2] = vw.z; T->ww[0] = ww.x; T->ww[1] = ww.y; T->ww[2] = ww.z;
     }
     // ob_hit / touch / tag are per-leg partial results: fold them over the legs here
-    int fl = (bad ? 1 : 0) | (ob_hit ? 2 : 0) | (touch_own ? 4 : 0) | (tag ? 8 : 0);
+    int fl = (bad ? tflag::bad : 0) | (ob_hit ? tflag::ob_hit : 0) | (touch_own ? tflag::touch_own : 0) | (tag ? tflag::tag : 0);
     fl |= __shfl_xor_sync(FULL, fl, 1); fl |= __shfl_xor_sync(FULL, fl, 2);
     if (l16 == 0) T->flags = fl;
     if (i == 0) {
@@ -1384,7 +1447,7 @@ __global__ void __launch_bounds__(LLQ16_BLOCK, LLQ16_MINB * 128 / LLQ16_BLOCK) l
     const int tenv_raw = blockIdx.x * EPB + tsrc;
     const float* tbase = s_env_dyn + tsrc * kEnvFloats;
     step_tail<ENV>(E, mc, P, M, &s_new[0][0], &s_hist[0][0], *reinterpret_cast<const TailState*>(tbase + (rowtab - linktab)),
-                        tbase + (envtab - linktab) + 44, obs2, obs2_ld, winner, seed, gid0, record, tel, tk, tenv_raw < N ? tenv_raw : N - 1, tval);
+                        tbase + (envtab - linktab) + envslot::act, obs2, obs2_ld, winner, seed, gid0, record, tel, tk, tenv_raw < N ? tenv_raw : N - 1, tval);
   }
   // ---- observation rows (history shift + new prop / action / future; EPMC / SEPMC: the 778 perception rays are cast while the row is
   // written): every warp of the CTA emits the rows of its own two envs, coalesced
